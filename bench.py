@@ -487,11 +487,51 @@ def run_extras(args, world, rank, dev, sweep, population, pop_local, timed_sweep
     return out
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, fitness, stats) -> None:
+    """What the timed path hands its caller after its last step, one float64 .npy per array: the fitness vector [individual]
+    and the lane stats [individual][symbol] of this rank's shard (trade_hash, a uint64, as its exact high and low 32-bit
+    halves).  Every value written is finite: an array holding inf or nan (the reference's Sortino ratio is +inf when a lane
+    has no downside deviation) is written with those entries as 0, and beside it <name>_nonfinite codes them as +1 (+inf),
+    -1 (-inf) or 2 (nan), 0 elsewhere.  Above DUMP_LIMIT_BYTES in all, a fixed seeded sample of individuals is written,
+    their indices in lane_index."""
+    import numpy as np
+    arrays = {"fitness": fitness}
+    for name, a in stats.items():
+        if name == "trade_hash":
+            arrays["trade_hash_hi"], arrays["trade_hash_lo"] = a >> np.uint64(32), a & np.uint64(0xFFFFFFFF)
+        else:
+            arrays[name] = a
+    for name, a in list(arrays.items()):
+        a = np.asarray(a, dtype=np.float64)
+        if not np.isfinite(a).all():
+            arrays[name + "_nonfinite"] = np.where(np.isnan(a), 2.0, np.where(np.isinf(a), np.sign(a), 0.0))
+            arrays[name] = np.where(np.isfinite(a), a, 0.0)
+    pop = len(fitness)
+    bytes_per_individual = 8 * (1 + sum(a.size // pop for a in arrays.values()))      # (+1: the lane_index entry)
+    if pop * bytes_per_individual > DUMP_LIMIT_BYTES:
+        idx = np.sort(np.random.default_rng(0).choice(pop, DUMP_LIMIT_BYTES // bytes_per_individual, replace=False))
+        arrays = {name: a[idx] for name, a in arrays.items()}
+        arrays["lane_index"] = idx
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
+def _positive_int(text: str) -> int:
+    n = int(text)
+    if n < 1:
+        raise argparse.ArgumentTypeError(f"must be at least 1, got {n}")
+    return n
+
+
 # --------------------------------------------------------------------------
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=_positive_int, default=10)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--pop-per-gpu", type=int, default=POP_PER_GPU)
@@ -502,6 +542,7 @@ def main():
     ap.add_argument("--cpu-baseline-only", action="store_true", help="(internal) print the cpu_baseline dict and exit")
     ap.add_argument("--reference-child", action="store_true", help="(internal) the worker of --impl reference")
     ap.add_argument("--mode", default="auto", choices=["auto", "fused", "chunked", "tiled"], help="sweep kernel path (auto = product default)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the fitness and lane stats of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
     if args.cpu_baseline_only:
         print(json.dumps(cpu_baseline_inline()), flush=True)
@@ -638,6 +679,8 @@ def main():
     evals_per_step_global = pop_global * S * N
     value = evals_per_step_global * args.steps / (ms_total * 1e-3)
     fit_random = fit_local.clone()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, fit_random.cpu().numpy(), sweep.lane_stats())
 
     # ---- parity spot check of the timed population (rank 0): 64 lanes against the C oracle ----
     parity = None
@@ -657,7 +700,7 @@ def main():
             f = out.cpu().numpy()
         return f, sw.h2d_bytes + mk.h2d_bytes, sw.d2h_bytes    # (the sweep reads close prices: the other OHLCV fields stay on the host)
 
-    e2e_steps = max(3, min(args.steps, 5))
+    e2e_steps = args.steps
     _phase("end-to-end leg")
     f_e2e, h2d, d2h = e2e_step()
     barrier()
@@ -750,13 +793,16 @@ def main():
             if "configs0_backtest" in cpu_baseline and not abandoned:
                 # the same configs[0] backtest through the GPU path (indicators, backtest_ref kernel, stats dict)
                 import asyncio
-                from ai_crypto_trader_b200.backtesting import StrategyTester
+                import tempfile
+                from ai_crypto_trader_b200.backtesting import HistoricalDataManager, StrategyTester
                 df0 = configs0_frame()
-                tester = StrategyTester(config={}, data_manager=None, results_dir=os.path.join(os.path.dirname(os.path.abspath(__file__)), "gpurun_out", "bench_results"), config_path=None)
-                asyncio.run(tester.backtest_frame(df0, "SYNUSDC"))
-                t0 = time.perf_counter()
-                st0 = asyncio.run(tester.backtest_frame(df0, "SYNUSDC"))
-                cpu_baseline["configs0_backtest"]["gpu_path_ms"] = (time.perf_counter() - t0) * 1e3
+                with tempfile.TemporaryDirectory(prefix="b200bt_bench_") as scratch:      # (the source tree may be read-only)
+                    tester = StrategyTester(config={}, data_manager=HistoricalDataManager(None, data_dir=os.path.join(scratch, "data")),
+                                            results_dir=os.path.join(scratch, "results"), config_path=None)
+                    asyncio.run(tester.backtest_frame(df0, "SYNUSDC"))
+                    t0 = time.perf_counter()
+                    st0 = asyncio.run(tester.backtest_frame(df0, "SYNUSDC"))
+                    cpu_baseline["configs0_backtest"]["gpu_path_ms"] = (time.perf_counter() - t0) * 1e3
                 cpu_baseline["configs0_backtest"]["gpu_trades"] = int(st0["total_trades"])
             line["cpu_baseline"] = cpu_baseline
         payload = (json.dumps(line) + "\n").encode()

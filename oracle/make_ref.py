@@ -26,7 +26,7 @@ FILES = ("services/strategy_evaluation.py", "services/genetic_algorithm.py", "co
 
 def place(force: bool = False) -> bool:
     """Copy FILES from the reference tree into oracle/_ref/ (build container).  -> True when oracle/_ref is complete."""
-    if (REFERENCE_ROOT / FILES[0]).exists():
+    if os.access(REFERENCE_ROOT / FILES[0], os.R_OK):     # (absent, or not readable by this user: nothing to place)
         for rel in FILES:
             dst = REF_DIR / rel
             if force or not dst.exists() or dst.stat().st_mtime < (REFERENCE_ROOT / rel).stat().st_mtime:

@@ -77,3 +77,38 @@ def test_claimed_stdout_carries_only_the_result_line():
     assert r.stdout == '{"value": 1}\n'
     for s in ("a python print", "a child of the shell", "a C library writing to fd 1"):
         assert s in r.stderr
+
+
+def test_dump_outputs_writes_float64_arrays_and_samples_above_the_limit(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: every array float64 and finite (inf / nan coded beside the array), trade_hash exact through
+    its two halves, a seeded sample above the cap."""
+    import numpy as np
+    import bench
+    rng = np.random.default_rng(1)
+    pop, S = 300, 3
+    fitness = rng.normal(size=pop)
+    sortino = rng.normal(size=(pop, S))
+    sortino[0, 0], sortino[5, 2], sortino[7, 1] = np.inf, -np.inf, np.nan
+    stats = {"score": rng.normal(size=(pop, S)), "sortino_ratio": sortino,
+             "trade_hash": rng.integers(0, 2**64, size=(pop, S), dtype=np.uint64)}
+    bench.dump_outputs(str(tmp_path / "all"), fitness, stats)
+    got = {p.stem: np.load(p) for p in (tmp_path / "all").glob("*.npy")}
+    assert set(got) == {"fitness", "score", "sortino_ratio", "sortino_ratio_nonfinite", "trade_hash_hi", "trade_hash_lo"}
+    assert all(a.dtype == np.float64 and np.isfinite(a).all() for a in got.values())
+    assert np.array_equal(got["fitness"], fitness) and np.array_equal(got["score"], stats["score"])
+    code = got["sortino_ratio_nonfinite"]
+    assert (code[0, 0], code[5, 2], code[7, 1]) == (1.0, -1.0, 2.0) and np.count_nonzero(code) == 3
+    finite = np.isfinite(sortino)
+    assert np.array_equal(got["sortino_ratio"][finite], sortino[finite]) and not got["sortino_ratio"][~finite].any()
+    hashes = (got["trade_hash_hi"].astype(np.uint64) << np.uint64(32)) | got["trade_hash_lo"].astype(np.uint64)
+    assert np.array_equal(hashes, stats["trade_hash"])
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 8 * (1 + 1 + 5 * S) * 100)        # room for 100 of the 300 individuals
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), fitness, stats)
+    a = {p.stem: np.load(p) for p in (tmp_path / "a").glob("*.npy")}
+    b = {p.stem: np.load(p) for p in (tmp_path / "b").glob("*.npy")}
+    assert sum(x.nbytes for x in a.values()) <= bench.DUMP_LIMIT_BYTES
+    idx = a["lane_index"].astype(np.int64)
+    assert len(idx) == 100 and np.array_equal(a["fitness"], fitness[idx]) and np.array_equal(a["score"], stats["score"][idx])
+    assert all(np.isfinite(x).all() for x in a.values())
+    assert set(a) == set(b) and all(np.array_equal(a[k], b[k]) for k in a)

@@ -41,11 +41,12 @@ def _check_against_reference(st, case, arrays, df):
 
 
 def test_strategy_tester_matches_reference(gpu, tmp_path):
-    from ai_crypto_trader_b200.backtesting import StrategyTester
+    from ai_crypto_trader_b200.backtesting import HistoricalDataManager, StrategyTester
     meta, arrays = load_bt_golden()
     for case in meta:
         df = bt_frame(case)
-        tester = StrategyTester(config={}, data_manager=None, results_dir=str(tmp_path / "res"), config_path=None)
+        tester = StrategyTester(config={}, data_manager=HistoricalDataManager(None, data_dir=str(tmp_path / "data")),
+                                results_dir=str(tmp_path / "res"), config_path=None)
         st = asyncio.run(tester.backtest_frame(df, "SYNUSDC"))
         c = tester.frame_constants
         assert c["signal"] == case["signal"] and c["strength"] == pytest.approx(unjson(case["strength"]), rel=1e-4, abs=1e-4)

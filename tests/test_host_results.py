@@ -1,15 +1,13 @@
 """ResultAnalyzer drop-in against the reference's own outputs (tests/golden/ra_reference.json, produced by executing
-backtesting/result_analyzer.py in make_golden.py), and the reference's run_backtest.py CLI driven through the
-drop-in package (build container only: needs /root/reference)."""
+backtesting/result_analyzer.py in make_golden.py), and the package entry points the reference's run_backtest.py CLI
+calls."""
 import json
 import os
-import subprocess
 import sys
 from pathlib import Path
 
-import pytest
 
-from conftest import GOLDEN, ROOT
+from conftest import GOLDEN
 
 
 def _strip(rs):
@@ -47,62 +45,53 @@ def test_result_analyzer_matches_reference_outputs(tmp_path):
     assert Path(ra.save_summary_report(s)).exists()
 
 
-REFERENCE = Path(os.environ.get("B200BT_REFERENCE_ROOT", "/root/reference"))
-
-_DRIVER = """
-import runpy, sys
-sys.path.insert(0, {repo!r})
-import ai_crypto_trader_b200.backtesting as b
-b.install_as_backtesting()
-sys.argv = ['run_backtest.py'] + {argv!r}
-runpy.run_path({script!r}, run_name='__main__')
-"""
-
-
-def _run_cli(cwd, argv):
-    code = _DRIVER.format(repo=str(ROOT), argv=argv, script=str(REFERENCE / "run_backtest.py"))
-    p = subprocess.run([sys.executable, "-c", code], cwd=cwd, capture_output=True, text=True, timeout=300)
-    out = p.stdout
-    start = out.find("\n{")                  # the CLI logs to stdout, then prints one JSON document
-    doc = json.loads(out[start:] if start >= 0 else out[out.find("{"):])
-    return p.returncode, doc, out
-
-
-@pytest.mark.skipif(not (REFERENCE / "run_backtest.py").exists(), reason="reference tree only exists in the build container")
-def test_reference_cli_runs_on_the_dropin(tmp_path):
-    """run_backtest.py (unmodified, run_backtest.py:11-12 imports resolved to the drop-in) `list`, `analyze`, `backtest`."""
+def test_cli_entry_points_on_the_dropin(tmp_path, monkeypatch):
+    """What the reference's run_backtest.py calls for `list`, `analyze` and `backtest`, with `import backtesting` resolved
+    to the drop-in and every object built with its default, working-directory-relative paths."""
+    import asyncio
     import numpy as np
     import pandas as pd
     from datetime import datetime
     from ai_crypto_trader_b200 import synth
-    from ai_crypto_trader_b200.backtesting import HistoricalDataManager
-    (tmp_path / "logs").mkdir()
+    import ai_crypto_trader_b200.backtesting as dropin
+    for name in ("backtesting", "backtesting.backtest_engine", "backtesting.data_manager", "backtesting.result_analyzer",
+                 "backtesting.strategy_tester"):
+        monkeypatch.setitem(sys.modules, name, None)                # (removed again after the test)
+    dropin.install_as_backtesting()
+    from backtesting import BacktestEngine, ResultAnalyzer
+    from backtesting.data_manager import HistoricalDataManager
+    assert BacktestEngine is dropin.BacktestEngine and HistoricalDataManager is dropin.HistoricalDataManager
+    monkeypatch.chdir(tmp_path)
     n = 3000
     d = synth.synth_symbol(0, n)
     idx = pd.date_range("2024-01-01", periods=n, freq="min")
     df = pd.DataFrame({k: d[k].astype(np.float64) for k in synth.FIELDS}, index=idx)
-    dm = HistoricalDataManager(None, data_dir=str(tmp_path / "backtesting" / "data"))
+    dm = HistoricalDataManager()
     dm.save_market_data("SYNUSDC", "1m", df, datetime(2024, 1, 1), datetime(2024, 1, 3))
-    rc, listing, _ = _run_cli(tmp_path, ["list"])
-    assert rc == 0 and listing == {"SYNUSDC": {"intervals": {"1m": {"start_date": "2024-01-01", "end_date": "2024-01-03", "days": 2}}}}
+    # list
+    dm = HistoricalDataManager()
+    assert dm.available_symbols() == ["SYNUSDC"] and dm.available_intervals("SYNUSDC") == ["1m"]
+    first, last = dm.get_data_range("SYNUSDC", "1m")
+    assert (first.strftime("%Y-%m-%d"), last.strftime("%Y-%m-%d"), (last - first).days) == ("2024-01-01", "2024-01-03", 2)
     # analyze: result files in the reference's layout (backtesting/results/*.json)
     ref = json.loads((GOLDEN / "ra_reference.json").read_text())
     res = tmp_path / "backtesting" / "results"
     res.mkdir(parents=True, exist_ok=True)
     for i, doc in enumerate(ref["documents"]):
         (res / f"result_{i:02d}.json").write_text(json.dumps(doc))
-    rc, summary, _ = _run_cli(tmp_path, ["analyze", "--symbols", "BTCUSDC", "--metric", "win_rate"])
-    assert rc == 0 and summary["total_results"] == 3 and summary["symbols"] == ["BTCUSDC"]
-    assert Path(tmp_path / summary["summary_path"]).exists() and Path(tmp_path / summary["comparison_chart"]).exists()
-    rc, summary, _ = _run_cli(tmp_path, ["analyze", "--results", str(res / "result_05.json"), str(res / "missing.json")])
-    assert rc == 0 and summary["total_results"] == 1 and summary["best_result"]["symbol"] == "ETHUSDC"
-    rc, none, _ = _run_cli(tmp_path, ["analyze", "--symbols", "NOPEUSDC"])
-    assert none == {"error": "No results found"}
+    ra = ResultAnalyzer()
+    results = ra.filter_results(symbol="BTCUSDC", interval=None)
+    summary = ra.generate_summary_report(results)
+    assert summary["total_results"] == 3 and summary["symbols"] == ["BTCUSDC"]
+    assert Path(ra.save_summary_report(summary)).exists() and Path(ra.compare_results(results, "win_rate")).exists()
+    picked = [r for r in (ra.load_results(str(res / "result_05.json")), ra.load_results(str(res / "missing.json"))) if r]
+    summary = ra.generate_summary_report(picked)
+    assert summary["total_results"] == 1 and summary["best_result"]["symbol"] == "ETHUSDC"
+    assert ra.filter_results(symbol="NOPEUSDC", interval=None) == []
     # backtest: on a CUDA box the stats of the GPU path; without a device the reference's error convention
     # ({'error': ...} per (symbol, interval), backtest_engine.py:125) -- never a CPU fallback
-    rc, bt, out = _run_cli(tmp_path, ["backtest", "--symbols", "SYNUSDC", "--intervals", "1m", "--start-date", "2024-01-01",
-                                      "--end-date", "2024-01-04", "--balance", "10000"])
-    assert rc == 0 and set(bt["SYNUSDC"]) == {"1m"}
+    bt = asyncio.run(BacktestEngine().run_multiple_backtests(["SYNUSDC"], ["1m"], datetime(2024, 1, 1), datetime(2024, 1, 4), 10000.0))
+    assert set(bt["SYNUSDC"]) == {"1m"}
     import torch
     if torch.cuda.is_available():
         assert bt["SYNUSDC"]["1m"]["initial_balance"] == 10000.0 and "total_trades" in bt["SYNUSDC"]["1m"]
