@@ -59,13 +59,22 @@ __host__ __device__ constexpr int64_t zone_fine_stride(int64_t N) { return ((N +
 // Evaluated as 100 U / (U + D) with ONE reciprocal: the two float64 divisions of the literal form were half of the RSI
 // bank kernel's instructions.  The forms agree to ~2e-14 absolute (1.5 ulp each), so they round to the same fp32 value
 // except on a ~1e-8 fraction of double-rounding ties -- below the 2e-6 the bank is tested at against float64 pandas.
-// A sum in the denormal range (thousands of flat bars) takes the literal form.
+// A D below the smallest normal double counts as 0: thousands of equal closes decay the averages into the subnormals, where
+// the serial recurrence either rounds them to exactly 0 (period 2) or leaves them stuck at the smallest subnormal, and
+// the scan's reassociated products round them differently; no price move is that small.  A sum still that small takes
+// the literal form.
 __device__ __forceinline__ float rsi_value(double U, double D) {
-    if (D == 0.0) return 100.0f;
+    if (D < 2.2250738585072014e-308) return 100.0f;
     const double S = U + D;
     if (S < 1e-290) return (float)(100.0 - 100.0 / (1.0 + U / D));
     return (float)((100.0 * U) * __drcp_rn(S));
 }
+
+// Seam states of RSI's Wilder averages over time tiles of `tile` bars (csrc/indicators.cu): seam[(sym P + p)(T - 1) + k]
+// = (U, D) after the last bar of tile k of row (sym, p), k < T - 1, T = ceil(N / tile); a kernel that starts tile k + 1
+// from it continues the serial recurrence exactly.
+int rsi_seam_states(const float* close, int S, int64_t N, int64_t ld, const int* periods_host, int P, int tile, double2* seam,
+                    cudaStream_t st);
 
 __device__ __forceinline__ double shfl_up_d(double v, int d) {
     return __shfl_up_sync(FULL, v, d);

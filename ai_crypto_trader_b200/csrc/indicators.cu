@@ -2,16 +2,20 @@
 //
 // Data layout: every series is a row of a row-major [S][N] fp32 matrix; a bank
 // is [S][P][N].  One CTA owns one (symbol, time-tile): it stages the close tile
-// (plus a warm-up halo) in shared memory once and its warps loop over the
+// in shared memory once and its warps loop over the
 // periods of the bank, so HBM sees 4 B/bar of input and 4 B/bar per output row.
 //
 // Linear recurrences (Wilder / EMA) are evaluated time-parallel: each lane
 // folds K consecutive bars into an affine map, the warp composes the 32 maps
 // with a shuffle scan, and the lanes replay their bars from the scanned state.
-// Tiles are made independent by starting the recurrence `halo` bars early from
-// a zero state: the forgotten state is attenuated by (1-alpha)^halo <= 2^-60,
-// i.e. below fp64 rounding, so the fp32 outputs match a serial float64
-// evaluation of the same recurrence.
+// Tiles are joined by an exact carry, not by a warm-up halo: RSI is the ratio
+// U / (U + D) of two Wilder averages, and a ratio keeps its value when both
+// terms decay, so a tile started from a zero state inside a run of equal closes
+// reads 100 where the serial recurrence keeps the RSI the run started with.
+// rsi_tile_end_kernel folds every tile but the last from a zero state into its
+// end state, rsi_seam_kernel composes those per row into the true state at
+// every seam (a warp scan over the tiles), and rsi_bank_kernel starts each tile
+// from that state.
 #include <math.h>
 #include "common.cuh"
 
@@ -24,8 +28,80 @@ constexpr int RSI_MAX_P = 128;
 
 struct RsiBankParams {
     int periods[RSI_MAX_P];
-    int halo[RSI_MAX_P];
 };
+
+// (U, D) after the last bar of tile k of row (sym, p), from a zero state at the tile's first bar; every tile but the last
+// of the series (those are whole).  One CTA per (tile, symbol), warps over the periods.  Lane l folds the 4-bar groups
+// l, l + 32, ... of the tile: acc = acc * om^128 + (group folded from 0); the tile's state is the sum of the lanes'
+// accumulators weighted by om^(4 (31 - l)).
+__global__ void __launch_bounds__(256)
+rsi_tile_end_kernel(const float* __restrict__ close, int64_t ld, const __grid_constant__ RsiBankParams prm, int P, int tile,
+                    double2* __restrict__ ends) {
+    extern __shared__ float s_c[];  // [tile + 1], s_c[i] = close[tile_start - 1 + i]
+    const int sym = blockIdx.y;
+    const int64_t tile_start = (int64_t)blockIdx.x * tile;
+    const float* row = close + (int64_t)sym * ld;
+    for (int i = threadIdx.x; i <= tile; i += blockDim.x) {
+        const int64_t t = tile_start - 1 + i;
+        s_c[i] = __ldg(row + (t < 0 ? 0 : t));          // diff = 0 at bar 0
+    }
+    __syncthreads();
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarp = blockDim.x >> 5;
+    for (int pi = warp; pi < P; pi += nwarp) {
+        const double alpha = 1.0 / (double)prm.periods[pi];
+        const double om = 1.0 - alpha;
+        const double a128 = pow(om, (double)RSI_STEP), wl = pow(om, (double)(RSI_K * (31 - lane)));
+        double accU = 0.0, accD = 0.0;
+        for (int base = 0; base < tile; base += RSI_STEP) {
+            const int i = base + lane * RSI_K;
+            double yU = 0.0, yD = 0.0;
+#pragma unroll
+            for (int j = 0; j < RSI_K; ++j) {
+                const double df = (double)s_c[i + j + 1] - (double)s_c[i + j];
+                yU = yU * om + alpha * (df > 0.0 ? df : 0.0);
+                yD = yD * om + alpha * (df < 0.0 ? -df : 0.0);
+            }
+            accU = accU * a128 + yU;
+            accD = accD * a128 + yD;
+        }
+        const double eU = warp_sum_d(accU * wl), eD = warp_sum_d(accD * wl);
+        if (lane == 0) ends[((int64_t)sym * P + pi) * gridDim.x + blockIdx.x] = make_double2(eU, eD);
+    }
+}
+
+// In place, one warp per row (sym, p) of `n_seam` entries: tile ends from a zero state -> the true (U, D) after the last
+// bar of each tile, C_k = m C_{k-1} + E_k with m = om^tile, 32 tiles per step of an affine shuffle scan.
+__global__ void __launch_bounds__(256)
+rsi_seam_kernel(const __grid_constant__ RsiBankParams prm, int P, int rows, int n_seam, int tile, double2* __restrict__ seam) {
+    const int lane = threadIdx.x & 31;
+    const int r = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (r >= rows) return;
+    const double om = 1.0 - 1.0 / (double)prm.periods[r % P];
+    double mp[5];
+#pragma unroll
+    for (int i = 0; i < 5; ++i) mp[i] = pow(om, (double)tile * (double)(1 << i));
+    const double ml = pow(om, (double)tile * (double)(lane + 1));
+    double2* s = seam + (int64_t)r * n_seam;
+    double cU = 0.0, cD = 0.0;
+    for (int k0 = 0; k0 < n_seam; k0 += 32) {
+        const int k = k0 + lane;
+        const double2 e = k < n_seam ? s[k] : make_double2(0.0, 0.0);
+        double yU = e.x, yD = e.y;
+#pragma unroll
+        for (int i = 0; i < 5; ++i) {
+            const double upU = shfl_up_d(yU, 1 << i), upD = shfl_up_d(yD, 1 << i);
+            if (lane >= (1 << i)) {
+                yU += mp[i] * upU;
+                yD += mp[i] * upD;
+            }
+        }
+        yU += ml * cU;
+        yD += ml * cD;
+        if (k < n_seam) s[k] = make_double2(yU, yD);
+        cU = shfl_d(yU, 31);
+        cD = shfl_d(yD, 31);
+    }
+}
 
 // ta.momentum.RSIIndicator semantics (binance_ml_strategy.py:112):
 //   diff = close.diff(1); up = max(diff,0); dn = max(-diff,0)  (bar 0: 0)
@@ -40,15 +116,15 @@ struct RsiBankParams {
 #endif
 __global__ void __launch_bounds__(256, B200BT_RSI_MIN_BLOCKS)
 rsi_bank_kernel(const float* __restrict__ close, int64_t N, int64_t ld,
-                const __grid_constant__ RsiBankParams prm, int P, int fill, int halo_max,
+                const __grid_constant__ RsiBankParams prm, int P, int fill, const double2* __restrict__ seam,
                 float* __restrict__ out, int vec_ok, float2* __restrict__ zc, float2* __restrict__ zf, int P_all, int p0) {
-    extern __shared__ float s_close[];  // [halo_max + RSI_TILE + 1], s_close[i] = close[s0 - 1 + i]
+    extern __shared__ float s_close[];  // [RSI_TILE + 1], s_close[i] = close[tile_start - 1 + i]
     const int sym = blockIdx.y;
     const int64_t tile_start = (int64_t)blockIdx.x * RSI_TILE;
     const int64_t tile_end = min(tile_start + (int64_t)RSI_TILE, N);
-    const int64_t s0 = max((int64_t)0, tile_start - halo_max);  // first bar staged (multiple of 4)
+    const int64_t s0 = tile_start;  // first bar staged
     const float* row = close + (int64_t)sym * ld;
-    const int n_stage = (int)(tile_start + RSI_TILE - s0) + 1;
+    const int n_stage = RSI_TILE + 1;
     for (int i = threadIdx.x; i < n_stage; i += blockDim.x) {
         int64_t t = s0 - 1 + i;
         t = t < 0 ? 0 : (t >= N ? N - 1 : t);  // clamp: diff = 0 outside the series
@@ -102,11 +178,13 @@ rsi_bank_kernel(const float* __restrict__ close, int64_t N, int64_t ld,
                 e >>= 1;
             }
         }
-        int64_t start = tile_start - prm.halo[pi];
-        start = start < s0 ? s0 : start;
-        start &= ~(int64_t)3;
-        double carryU = 0.0, carryD = 0.0;
-        for (int64_t base = start; base < tile_end; base += RSI_STEP) {
+        double carryU = 0.0, carryD = 0.0;     // the true state before the tile's first bar (rsi_seam_kernel)
+        if (blockIdx.x > 0) {
+            const double2 c = seam[((int64_t)sym * P + pi) * (gridDim.x - 1) + blockIdx.x - 1];
+            carryU = c.x;
+            carryD = c.y;
+        }
+        for (int64_t base = tile_start; base < tile_end; base += RSI_STEP) {
             const int64_t t = base + lane * RSI_K;
             const int si = (int)(t - s0);  // s_close[si] = close[t-1]
             double x[RSI_K + 1];
@@ -145,7 +223,7 @@ rsi_bank_kernel(const float* __restrict__ close, int64_t N, int64_t ld,
                 D = D * om + alpha * d[j];
                 r[j] = rsi_value(U, D);
             }
-            const bool mine = t >= tile_start && t < tile_end;
+            const bool mine = t < tile_end;
             if (mine) {
                 if (vec_ok && t + RSI_K <= tile_end) {
                     *reinterpret_cast<float4*>(orow + t) = make_float4(r[0], r[1], r[2], r[3]);
@@ -156,7 +234,7 @@ rsi_bank_kernel(const float* __restrict__ close, int64_t N, int64_t ld,
                 }
             }
             if (zcr) {
-                // this lane's four bars are one 4-bar group, eight lanes (start is a multiple of 32) one 32-bar block
+                // this lane's four bars are one 4-bar group, eight lanes (the tile start is a multiple of 32) one 32-bar block
                 float lo = qnan, hi = qnan;
 #pragma unroll
                 for (int j = 0; j < RSI_K; ++j)
@@ -165,7 +243,7 @@ rsi_bank_kernel(const float* __restrict__ close, int64_t N, int64_t ld,
 #pragma unroll
                 for (int m = 1; m < 8; m <<= 1) { lo = fminf(lo, __shfl_xor_sync(FULL, lo, m)); hi = fmaxf(hi, __shfl_xor_sync(FULL, hi, m)); }
                 const int64_t tb = t & ~(int64_t)31;
-                if ((lane & 7) == 0 && tb >= tile_start && tb < tile_end) zcr[tb >> 5] = make_float2(lo, hi);
+                if ((lane & 7) == 0 && tb < tile_end) zcr[tb >> 5] = make_float2(lo, hi);
             }
         }
         if (zcr && last_tile) {
@@ -201,11 +279,24 @@ rsi_bank_kernel(const float* __restrict__ close, int64_t N, int64_t ld,
     }
 }
 
-static int halo_for_alpha(double alpha) {
-    // (1-alpha)^L <= 2^-60
-    double L = ceil(60.0 * log(2.0) / -log1p(-alpha));
-    if (!(L < 1e9)) L = 1e9;
-    return ((int)L + 31) & ~31;     // a multiple of 32: the scan then starts on a zone-block boundary
+// Seam states of the Wilder averages of RSI over tiles of `tile` bars (a multiple of RSI_STEP): seam[(sym P + p)(T - 1) + k]
+// = (U, D) after the last bar of tile k, k < T - 1, T = ceil(N / tile).  Nothing to do for a single tile.
+int rsi_seam_states(const float* close, int S, int64_t N, int64_t ld, const int* periods_host, int P, int tile, double2* seam,
+                    cudaStream_t st) {
+    const int64_t T = (N + tile - 1) / tile;
+    if (T < 2) return B200BT_OK;
+    B200BT_REQUIRE(P <= RSI_MAX_P && tile % RSI_STEP == 0, B200BT_ELIMIT, "rsi seam states: bad tiling");
+    RsiBankParams prm;
+    for (int i = 0; i < P; ++i) prm.periods[i] = periods_host[i];
+    const size_t smem = (size_t)(tile + 1) * sizeof(float);
+    cudaError_t e = cudaFuncSetAttribute(rsi_tile_end_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return cuda_status(e, "rsi seam states: cudaFuncSetAttribute");
+    rsi_tile_end_kernel<<<dim3((unsigned)(T - 1), (unsigned)S), 256, smem, st>>>(close, ld, prm, P, tile, seam);
+    B200BT_LAUNCH_CHECK("rsi tile end launch");
+    const int rows = S * P;
+    rsi_seam_kernel<<<(unsigned)((rows + 7) / 8), 256, 0, st>>>(prm, P, rows, (int)(T - 1), tile, seam);
+    B200BT_LAUNCH_CHECK("rsi seam launch");
+    return B200BT_OK;
 }
 
 }  // namespace b200bt
@@ -228,37 +319,49 @@ extern "C" int b200bt_rsi_bank_zones(const float* close, int S, int64_t N, int64
     return rsi_bank_impl(close, S, N, ld, periods_host, P, 1, out, zones, S_total, sym0, stream);
 }
 
+static int rsi_bank_launches(const float* close, int S, int64_t N, int64_t ld, const int* periods_host, int P, int fill,
+                             float* out, float* zones, int S_total, int sym0, double2* seam, cudaStream_t st) {
+    const bool vec_ok = (N % 4 == 0) && (((uintptr_t)out & 15) == 0);
+    const size_t smem = (size_t)(RSI_TILE + 4) * sizeof(float);
+    for (int p0 = 0; p0 < P; p0 += RSI_MAX_P) {
+        const int pc = (P - p0) < RSI_MAX_P ? (P - p0) : RSI_MAX_P;
+        RsiBankParams prm;
+        for (int i = 0; i < pc; ++i) prm.periods[i] = periods_host[p0 + i];
+        int rc = rsi_seam_states(close, S, N, ld, periods_host + p0, pc, RSI_TILE, seam, st);
+        if (rc) return rc;
+        dim3 grid((unsigned)((N + RSI_TILE - 1) / RSI_TILE), (unsigned)S);
+        // the launch writes rows [p0, p0+pc) of every symbol: pass the full-P row pitch via (P, pi offset)
+        float2* zc = zones ? (float2*)zones + (int64_t)sym0 * (P + 1) * zone_row_stride(N) : nullptr;
+        float2* zf = zones ? (float2*)zones + (int64_t)S_total * (P + 1) * zone_row_stride(N) + (int64_t)sym0 * (P + 1) * zone_fine_stride(N) : nullptr;
+        rsi_bank_kernel<<<grid, 256, smem, st>>>(close, N, ld, prm, pc, fill, seam,
+                                                  out + (int64_t)p0 * N, vec_ok ? 1 : 0, zc, zf, P, p0);
+        B200BT_LAUNCH_CHECK("rsi_bank launch");
+    }
+    return B200BT_OK;
+}
+
 static int rsi_bank_impl(const float* close, int S, int64_t N, int64_t ld, const int* periods_host, int P, int fill,
                          float* out, float* zones, int S_total, int sym0, b200bt_stream_t stream) {
     B200BT_REQUIRE(close && out && periods_host, B200BT_EINVAL, "rsi_bank: null pointer");
     B200BT_REQUIRE(S > 0 && N > 0 && P > 0 && ld >= N, B200BT_EINVAL, "rsi_bank: bad sizes S=%d N=%lld P=%d", S, (long long)N, P);
     B200BT_REQUIRE(P <= RSI_MAX_P, B200BT_ELIMIT, "rsi_bank: at most %d periods per call", RSI_MAX_P);
+    for (int i = 0; i < P; ++i)
+        B200BT_REQUIRE(periods_host[i] >= 1 && periods_host[i] <= RSI_TILE, B200BT_ELIMIT, "rsi_bank: window %d outside [1,%d]",
+                       periods_host[i], RSI_TILE);
     int rc = check_device();
     if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
-    const bool vec_ok = (N % 4 == 0) && (((uintptr_t)out & 15) == 0);
-    for (int p0 = 0; p0 < P; p0 += RSI_MAX_P) {
-        const int pc = (P - p0) < RSI_MAX_P ? (P - p0) : RSI_MAX_P;
-        RsiBankParams prm;
-        int halo_max = 0;
-        for (int i = 0; i < pc; ++i) {
-            int w = periods_host[p0 + i];
-            B200BT_REQUIRE(w >= 1 && w <= RSI_TILE, B200BT_ELIMIT, "rsi_bank: window %d outside [1,%d]", w, RSI_TILE);
-            prm.periods[i] = w;
-            prm.halo[i] = (w == 1) ? 4 : halo_for_alpha(1.0 / w);
-            if (prm.halo[i] > halo_max) halo_max = prm.halo[i];
-        }
-        const size_t smem = (size_t)(halo_max + RSI_TILE + 4) * sizeof(float);
-        B200BT_REQUIRE(smem <= 200 * 1024, B200BT_ELIMIT, "rsi_bank: window too long for the shared-memory tile");
-        cudaError_t e = cudaFuncSetAttribute(rsi_bank_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return cuda_status(e, "rsi_bank: cudaFuncSetAttribute");
-        dim3 grid((unsigned)((N + RSI_TILE - 1) / RSI_TILE), (unsigned)S);
-        // the launch writes rows [p0, p0+pc) of every symbol: pass the full-P row pitch via (P, pi offset)
-        float2* zc = zones ? (float2*)zones + (int64_t)sym0 * (P + 1) * zone_row_stride(N) : nullptr;
-        float2* zf = zones ? (float2*)zones + (int64_t)S_total * (P + 1) * zone_row_stride(N) + (int64_t)sym0 * (P + 1) * zone_fine_stride(N) : nullptr;
-        rsi_bank_kernel<<<grid, 256, smem, st>>>(close, N, ld, prm, pc, fill, halo_max,
-                                                  out + (int64_t)p0 * N, vec_ok ? 1 : 0, zc, zf, P, p0);
-        B200BT_LAUNCH_CHECK("rsi_bank launch");
+    // seam states of one launch's rows, stream-ordered: concurrent calls on other streams get their own
+    const int64_t T = (N + RSI_TILE - 1) / RSI_TILE;
+    double2* seam = nullptr;
+    if (T > 1) {
+        cudaError_t e = cudaMallocAsync((void**)&seam, (size_t)S * (P < RSI_MAX_P ? P : RSI_MAX_P) * (T - 1) * sizeof(double2), st);
+        if (e != cudaSuccess) return cuda_status(e, "rsi_bank: seam states");
     }
-    return B200BT_OK;
+    rc = rsi_bank_launches(close, S, N, ld, periods_host, P, fill, out, zones, S_total, sym0, seam, st);
+    if (seam) {
+        cudaError_t e = cudaFreeAsync(seam, st);
+        if (!rc && e != cudaSuccess) rc = cuda_status(e, "rsi_bank: seam states");
+    }
+    return rc;
 }

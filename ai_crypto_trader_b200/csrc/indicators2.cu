@@ -11,7 +11,9 @@
 // the reference's `_handle_nan_values` policy, resolved by the nanfill kernels
 // (ffill -> bfill -> 0).
 //   * exponential recurrences (EMA, MACD, ATR): time-parallel affine warp scan, tiles made
-//     independent by a warm-up halo that attenuates the unknown state below 2^-60;
+//     independent by a warm-up halo that attenuates the unknown state below 2^-60 (RSI, a
+//     ratio of two such averages that a halo cannot make exact, is carried across the seams:
+//     rsi_seam_states, csrc/indicators.cu);
 //   * window sums (SMA, Bollinger, VWAP, %D): fp64 prefix sums of tile-offset values in
 //     shared memory, window sum = difference of two prefixes;
 //   * window extrema (stochastic, Williams, Ichimoku): direct scan of the window in shared
@@ -673,23 +675,28 @@ __device__ __forceinline__ void lead_fill(const LeadFill& lf, int sym, int64_t N
 
 __global__ void __launch_bounds__(64)
 analyzer_a_kernel(const float* __restrict__ x, int64_t N, int64_t ld, int fast, int slow, int sign, int halo_ema, int halo_sig,
-                  int w_rsi, int halo_rsi, float* __restrict__ o_ef, float* __restrict__ o_es, float* __restrict__ o_line,
-                  float* __restrict__ o_sig, float* __restrict__ o_diff, float* __restrict__ o_rsi, const LeadFill lf) {
+                  int w_rsi, const double2* __restrict__ rsi_seam, float* __restrict__ o_ef, float* __restrict__ o_es,
+                  float* __restrict__ o_line, float* __restrict__ o_sig, float* __restrict__ o_diff, float* __restrict__ o_rsi, const LeadFill lf) {
     extern __shared__ double s_line[];
     const int sym = blockIdx.y, lane = threadIdx.x & 31;
     const int64_t tile_start = (int64_t)blockIdx.x * IND_TILE, tile_end = min(tile_start + (int64_t)IND_TILE, N);
     if (threadIdx.x < 32) {
         macd_tile(x, N, ld, fast, slow, sign, halo_ema, halo_sig, o_line, o_sig, o_diff, o_ef, o_es, s_line, sym, tile_start);
     } else {
-        // RSI (ta.momentum.RSIIndicator, :112): Wilder averages of the up / down moves, y0 = x0 (both 0 at bar 0)
+        // RSI (ta.momentum.RSIIndicator, :112): Wilder averages of the up / down moves, y0 = x0 (both 0 at bar 0), started
+        // from their true state at the tile's first bar
         const float* row = x + (int64_t)sym * ld;
         constexpr int K = 4;
         const double alpha = 1.0 / (double)w_rsi;
         AffineScan<K> sc;
         sc.init(1.0 - alpha, lane);
-        const int64_t start = max((int64_t)0, tile_start - halo_rsi) & ~(int64_t)3;
         double cu = 0.0, cd = 0.0;
-        for (int64_t base = start; base < tile_end; base += 32 * K) {
+        if (blockIdx.x > 0) {
+            const double2 c = rsi_seam[(int64_t)sym * (gridDim.x - 1) + blockIdx.x - 1];
+            cu = c.x;
+            cd = c.y;
+        }
+        for (int64_t base = tile_start; base < tile_end; base += 32 * K) {
             const int64_t t = base + lane * K;
             double xs[K + 1], bu[K], bd[K], yu[K], yd[K];
 #pragma unroll
@@ -708,7 +715,7 @@ analyzer_a_kernel(const float* __restrict__ x, int64_t N, int64_t ld, int fast, 
             sc.run(bd, cd, yd, lane);
 #pragma unroll
             for (int j = 0; j < K; ++j)
-                if (t + j >= tile_start && t + j < tile_end) {
+                if (t + j < tile_end) {
                     o_rsi[(int64_t)sym * N + t + j] = (t + j >= w_rsi - 1) ? rsi_value(yu[j], yd[j]) : nanf32();
                 }
         }
@@ -1097,14 +1104,19 @@ extern "C" int b200bt_vwap(const float* high, const float* low, const float* clo
 }
 
 // TechnicalAnalyzer._calculate_all_indicators for S symbols: three fused launches + one batched NaN-policy call.
+// The workspace holds the RSI column's seam states (S x (tiles - 1) double2) during launch A, then the NaN policy's tile
+// summaries.
 extern "C" int64_t b200bt_analyzer_workspace_floats(int S, int64_t N) {
-    return b200bt_nanfill_workspace_floats((int64_t)5 * S, N);
+    const int64_t seam = (int64_t)4 * S * ((N + IND_TILE - 1) / IND_TILE - 1);
+    const int64_t nf = b200bt_nanfill_workspace_floats((int64_t)5 * S, N);
+    return seam > nf ? seam : nf;
 }
 
 extern "C" int b200bt_analyzer(const float* high, const float* low, const float* close, const float* volume, int S, int64_t N,
                                int64_t ld, float* cols, float* workspace, b200bt_stream_t stream) {
     B200BT_REQUIRE(high && low && close && volume && cols && workspace, B200BT_EINVAL, "analyzer: null pointer");
     IND_COMMON_CHECKS("analyzer");
+    B200BT_REQUIRE(((uintptr_t)workspace & 15) == 0, B200BT_EINVAL, "analyzer: workspace must be 16-byte aligned");
     cudaStream_t st = (cudaStream_t)stream;
     const int64_t plane = (int64_t)S * N;
     auto col = [&](int c) { return cols + (int64_t)c * plane; };
@@ -1114,7 +1126,9 @@ extern "C" int b200bt_analyzer(const float* high, const float* low, const float*
     // A: close -> ema_12, ema_26, macd, macd_signal, macd_diff, rsi
     {
         const int halo_ema = halo_for(1.0 - 2.0 / ((double)slow + 1.0)), halo_sig = halo_for(1.0 - 2.0 / ((double)sign + 1.0));
-        const int halo_rsi = halo_for(((double)w_rsi - 1.0) / (double)w_rsi);
+        double2* rsi_seam = reinterpret_cast<double2*>(workspace);
+        int rc = rsi_seam_states(close, S, N, ld, &w_rsi, 1, IND_TILE, rsi_seam, st);
+        if (rc) return rc;
         const size_t smem = (size_t)(halo_sig + IND_TILE + 8) * sizeof(double);
         cudaError_t e = cudaFuncSetAttribute(analyzer_a_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return cuda_status(e, "analyzer: cudaFuncSetAttribute");
@@ -1123,7 +1137,7 @@ extern "C" int b200bt_analyzer(const float* high, const float* low, const float*
         const int fs[6] = {fast - 1, slow - 1, slow - 1, slow - 1 + sign - 1, slow - 1 + sign - 1, w_rsi - 1};
         lf.n = 6;
         for (int i = 0; i < 6; ++i) { lf.col[i] = col(cs[i]); lf.first[i] = fs[i]; }
-        analyzer_a_kernel<<<ind_grid(N, S), 64, smem, st>>>(close, N, ld, fast, slow, sign, halo_ema, halo_sig, w_rsi, halo_rsi,
+        analyzer_a_kernel<<<ind_grid(N, S), 64, smem, st>>>(close, N, ld, fast, slow, sign, halo_ema, halo_sig, w_rsi, rsi_seam,
                                                            col(B200BT_COL_EMA_12), col(B200BT_COL_EMA_26), col(B200BT_COL_MACD),
                                                            col(B200BT_COL_MACD_SIGNAL), col(B200BT_COL_MACD_DIFF), col(B200BT_COL_RSI), lf);
         B200BT_LAUNCH_CHECK("analyzer A launch");

@@ -64,7 +64,7 @@ int b200bt_rsi_bank(const float* close, int S, int64_t N, int64_t ld,
  * fused launches (close -> EMA / MACD / RSI; close -> SMA / Bollinger; high, low, close, volume -> stochastic / Williams %R /
  * Ichimoku / ATR / VWAP) plus one batched NaN-policy call, with the reference's windows (20/50/200, 12/26/9, 9/26/52, 14, 14/3,
  * 14, 20 x 2.0, 14, 14).  cols: [B200BT_ANALYZER_COLUMNS][S][N] fp32 (device, out), column c at cols + c * S * N in the order
- * below; workspace: b200bt_analyzer_workspace_floats(S, N) floats (device). */
+ * below; workspace: b200bt_analyzer_workspace_floats(S, N) floats (device, 16-byte aligned). */
 enum b200bt_analyzer_column {
     B200BT_COL_SMA_20 = 0, B200BT_COL_SMA_50, B200BT_COL_SMA_200, B200BT_COL_EMA_12, B200BT_COL_EMA_26, B200BT_COL_MACD,
     B200BT_COL_MACD_SIGNAL, B200BT_COL_MACD_DIFF, B200BT_COL_ICHIMOKU_A, B200BT_COL_ICHIMOKU_B, B200BT_COL_RSI, B200BT_COL_BB_HIGH,

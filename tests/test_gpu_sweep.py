@@ -486,7 +486,7 @@ def test_zone_rows_written_with_the_bank_equal_the_zone_map_kernel(torch_cuda, n
     import ctypes as C
     from ai_crypto_trader_b200 import _lib, synth
     from ai_crypto_trader_b200.sweep import rsi_bank
-    S, periods = 3, [2, 5, 14, 30]
+    S, periods = 3, [1, 2, 5, 14, 30]
     P = len(periods)
     close = torch.from_numpy(synth.synth_ohlcv(S, n_bars, first_symbol=3)[3]).cuda()
     nz = int(_lib.load().b200bt_zone_map_floats(P, S, n_bars))
