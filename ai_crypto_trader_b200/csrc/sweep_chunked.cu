@@ -14,22 +14,51 @@
 //                   THREAD per (individual, symbol, chunk) (b200bt_sweep_tiled, see "thread-per-lane scan").
 //                   Events -> blocks of a global pool (bump allocator, singly linked per chunk), plus the
 //                   chunk's assumed state at T_c and its end state.
-//   verify / repair lane_repair_kernel: one warp per lane walks the chunk boundaries in time order and re-scans a chunk
-//                   whose assumed state differs from its predecessor's end state (chunk_scan_item<REPAIR>: from the true
-//                   state, until the trajectory meets the recorded one; the rest of the recorded chain is spliced on).
-//                   A bounded pass on the critical path, an unbounded one beside the metrics kernels (finish_chunks).
+//   verify / repair a chunk whose assumed state differs from its predecessor's end state is re-scanned from the true
+//                   state until the trajectory meets the recorded one; the rest of the recorded chain is spliced on
+//                   (chunk_scan_item<REPAIR>).  chunk_repair_kernel: one warp per chunk, on the critical path;
+//                   lane_repair_kernel: one warp per lane, in time order, beside the metrics kernels (finish_chunks).
 //   metrics kernels one warp per (individual, symbol, chunk) again (see "metrics, chunk-parallel" below), then
 //                   one thread per (individual, symbol) checks end state of chunk c-1 == assumed state
 //                   of chunk c for every boundary and merges the chunks' partial metrics.
 // A lane with any mismatching boundary is flagged; the host re-evaluates flagged lanes with the
 // fused (serial) kernel, so results never depend on the speculation being right.
-#include <stdlib.h>
+#include <stddef.h>
 #include "sweep_dev.cuh"
 
 namespace b200bt {
 
 constexpr int CK_BLOCK = 256;   // events per pool block
 constexpr unsigned EVENT_BAR_MASK = ~(B200BT_EVENT_EXIT | B200BT_EVENT_SELL);   // event word = bar | flags
+
+// Segment (one chunk of one lane) vocabulary.  A chunk's state at a bar is (position side, entry bar), the entry bar -1
+// when flat.  A chunk that LOST its events (full pool, a tile that did not arrive, a warp not packed for the thread-per-lane
+// scan) has no chain: its count is SEG_LOST, which sends it to the repair pass or its lane to the exact fallback.
+constexpr unsigned SEG_LOST = 0xffffffffu;
+
+__device__ __forceinline__ int2 seg_state(int pos, int entry_bar) { return make_int2(pos, pos != 0 ? entry_bar : -1); }
+
+// The event pool and the per-segment tables, shared by every kernel of the time-chunked sweep.
+struct SegTables {
+    uint2* pool; int pool_blocks; int* next; unsigned* alloc; int* overflow;    // [pool_blocks][CK_BLOCK] events, chain links
+    int* seg_first; unsigned* seg_count; int2* seg_in; int2* seg_out;          // [segs]: first block, events, assumed / end state
+};
+
+__device__ __forceinline__ void mark_lost(const SegTables& T, int seg) {
+    T.seg_in[seg] = seg_state(0, 0);
+    T.seg_out[seg] = seg_state(0, 0);
+    T.seg_count[seg] = SEG_LOST;
+}
+
+// Appends a pool block to the chain of segment `seg`, whose last block is `cur_block` (-1: none yet).  -> the block, or
+// -1 when the pool is exhausted (the overflow flag is raised; the caller drops the chunk's further events).
+__device__ __forceinline__ int pool_append(const SegTables& T, int seg, int cur_block) {
+    const int b = (int)atomicAdd(T.alloc, 1u);
+    if (b >= T.pool_blocks) { atomicExch(T.overflow, 1); return -1; }
+    T.next[b] = -1;
+    if (cur_block < 0) T.seg_first[seg] = b; else T.next[cur_block] = b;
+    return b;
+}
 
 struct ChunkScanArgs {
     const float* price; int64_t ld_price;
@@ -38,8 +67,7 @@ struct ChunkScanArgs {
     const b200bt_individual* indiv;
     const b200bt_chunk_item* items; int n_items; int n_seg;   // n_seg = segments per symbol
     int warm;
-    uint2* pool; int pool_blocks; int* next; unsigned* alloc;
-    int* seg_first; unsigned* seg_count; int2* seg_in; int2* seg_out; int* overflow;
+    SegTables T;
     const int32_t* n_chunks;
     unsigned char* redo;  // repair pass of the overlapped tail: individuals whose metrics must be recomputed
 };
@@ -83,7 +111,7 @@ __device__ __forceinline__ bool chunk_scan_item(const ChunkScanArgs& A, const b2
     unsigned qtail = 0;
     if (REPAIR) {
         // true state at T0 = end state of the preceding chunk (position side, entry bar -> entry price)
-        const int2 z = A.seg_out[seg - 1];
+        const int2 z = A.T.seg_out[seg - 1];
         if (z.x != 0) {
             const float e = __ldg(pr + z.y);
             m.pos = z.x; m.e = e; m.entry_bar = z.y;
@@ -104,11 +132,11 @@ __device__ __forceinline__ bool chunk_scan_item(const ChunkScanArgs& A, const b2
     unsigned old_left = 0;
     bool old_ok = false, spliced = false;
     if (REPAIR) {
-        const unsigned oc = A.seg_count[seg];
-        const int2 oin = A.seg_in[seg];
-        old_ok = oc != 0xffffffffu;     // (a chunk whose events were dropped has no chain to splice)
+        const unsigned oc = A.T.seg_count[seg];
+        const int2 oin = A.T.seg_in[seg];
+        old_ok = oc != SEG_LOST;     // (a chunk whose events were dropped has no chain to splice)
         old_left = old_ok ? oc : 0u;
-        old_block = A.seg_first[seg];
+        old_block = A.T.seg_first[seg];
         old_pos = oin.x; old_ebar = oin.x != 0 ? oin.y : -1;
     }
 
@@ -117,19 +145,12 @@ __device__ __forceinline__ bool chunk_scan_item(const ChunkScanArgs& A, const b2
     auto flush = [&](int cnt) {
         if (fill == CK_BLOCK && !dead) {
             int b = 0;
-            if (lane == 0) {
-                b = (int)atomicAdd(A.alloc, 1u);
-                if (b >= A.pool_blocks) { atomicExch(A.overflow, 1); b = -1; }
-                else {
-                    A.next[b] = -1;
-                    if (cur_block < 0) A.seg_first[seg] = b; else A.next[cur_block] = b;
-                }
-            }
+            if (lane == 0) b = pool_append(A.T, seg, cur_block);
             b = __shfl_sync(FULL, b, 0);
             if (b < 0) dead = 1; else { cur_block = b; fill = 0; }
         }
         if (!dead) {
-            if (lane < cnt) A.pool[(int64_t)cur_block * CK_BLOCK + fill + lane] = ws->evq[(qtail + lane) & (SW_EVQ - 1)];
+            if (lane < cnt) A.T.pool[(int64_t)cur_block * CK_BLOCK + fill + lane] = ws->evq[(qtail + lane) & (SW_EVQ - 1)];
             fill += 32;   // only the last flush of a chunk is partial
         }
         qtail += cnt;
@@ -181,20 +202,20 @@ __device__ __forceinline__ bool chunk_scan_item(const ChunkScanArgs& A, const b2
         cp_async_wait<SW_STAGES - 1>();
         __syncwarp();
         const bool emit = g * G >= T0;
-        if (g * G == T0 && lane == 0) A.seg_in[seg] = make_int2(m.pos, m.pos != 0 ? m.entry_bar : -1);
+        if (g * G == T0 && lane == 0) A.T.seg_in[seg] = seg_state(m.pos, m.entry_bar);
         if (REPAIR && old_ok && g > g_begin) {
             // state of the recorded trajectory before bar tb = g * G: consume its events with bar < tb
             const unsigned tb = (unsigned)(g * G);
             while (old_left) {
                 const int n_here = (int)min(min(32u, old_left), (unsigned)(CK_BLOCK - old_idx));
-                const unsigned word = lane < n_here ? A.pool[(int64_t)old_block * CK_BLOCK + old_idx + lane].x : 0xffffffffu;
+                const unsigned word = lane < n_here ? A.T.pool[(int64_t)old_block * CK_BLOCK + old_idx + lane].x : 0xffffffffu;
                 const int k = __popc(__ballot_sync(FULL, lane < n_here && (word & EVENT_BAR_MASK) < tb));    // (bars ascend: a prefix)
                 if (k) {
                     const unsigned last = __shfl_sync(FULL, word, k - 1);
                     old_pos = (last & B200BT_EVENT_EXIT) ? 0 : ((last & B200BT_EVENT_SELL) ? -1 : 1);
                     old_ebar = (last & B200BT_EVENT_EXIT) ? -1 : (int)(last & EVENT_BAR_MASK);
                     old_idx += k; old_left -= (unsigned)k;
-                    if (old_idx == CK_BLOCK && old_left) { old_block = A.next[old_block]; old_idx = 0; }
+                    if (old_idx == CK_BLOCK && old_left) { old_block = A.T.next[old_block]; old_idx = 0; }
                 }
                 if (k < n_here) break;
             }
@@ -203,10 +224,10 @@ __device__ __forceinline__ bool chunk_scan_item(const ChunkScanArgs& A, const b2
                 // re-scanned events (the chunk's end state, and with it every later chunk, stands as recorded)
                 while (old_left) {
                     const int n_here = (int)min(min(32u, old_left), (unsigned)(CK_BLOCK - old_idx));
-                    if (lane < n_here) ws->evq[(m.qhead + lane) & (SW_EVQ - 1)] = A.pool[(int64_t)old_block * CK_BLOCK + old_idx + lane];
+                    if (lane < n_here) ws->evq[(m.qhead + lane) & (SW_EVQ - 1)] = A.T.pool[(int64_t)old_block * CK_BLOCK + old_idx + lane];
                     m.qhead += (unsigned)n_here;
                     old_idx += n_here; old_left -= (unsigned)n_here;
-                    if (old_idx == CK_BLOCK && old_left) { old_block = A.next[old_block]; old_idx = 0; }
+                    if (old_idx == CK_BLOCK && old_left) { old_block = A.T.next[old_block]; old_idx = 0; }
                     __syncwarp();
                     while (m.qhead - qtail >= 32) flush(32);
                     __syncwarp();
@@ -237,9 +258,9 @@ __device__ __forceinline__ bool chunk_scan_item(const ChunkScanArgs& A, const b2
     }
     cp_async_wait<0>();
     if (lane == 0 && !spliced) {
-        const int2 st = make_int2(m.pos, m.pos != 0 ? m.entry_bar : -1);
-        A.seg_out[seg] = st;
-        if (T0 >= T1) A.seg_in[seg] = st;   // empty chunk: its assumed state is the state after the warm-up
+        const int2 st = seg_state(m.pos, m.entry_bar);
+        A.T.seg_out[seg] = st;
+        if (T0 >= T1) A.T.seg_in[seg] = st;   // empty chunk: its assumed state is the state after the warm-up
     }
     if (!spliced && item.chunk == item.n_chunks - 1 && m.pos != 0) {
         // force-close at the last bar (:849-876)
@@ -250,7 +271,7 @@ __device__ __forceinline__ bool chunk_scan_item(const ChunkScanArgs& A, const b2
     }
     __syncwarp();
     while (m.qhead != qtail) flush((int)min(32u, m.qhead - qtail));
-    if (lane == 0) A.seg_count[seg] = dead ? 0xffffffffu : m.qhead;
+    if (lane == 0) A.T.seg_count[seg] = dead ? SEG_LOST : m.qhead;
     __syncwarp();
     return spliced;      // REPAIR: the chunk's recorded end state stands
 }
@@ -291,8 +312,8 @@ chunk_repair_kernel(const ChunkScanArgs A, unsigned* __restrict__ work) {
         const b200bt_chunk_item item = A.items[it];
         if (item.chunk == 0) continue;
         const int seg = sym * A.n_seg + item.segment;
-        const int2 a = A.seg_in[seg], z = A.seg_out[seg - 1];
-        if ((a.x != z.x || a.y != z.y) && A.seg_count[seg - 1] != 0xffffffffu) chunk_scan_item<VEC16, true>(A, item, sym, ws);
+        const int2 a = A.T.seg_in[seg], z = A.T.seg_out[seg - 1];
+        if ((a.x != z.x || a.y != z.y) && A.T.seg_count[seg - 1] != SEG_LOST) chunk_scan_item<VEC16, true>(A, item, sym, ws);
     }
 }
 
@@ -317,18 +338,18 @@ lane_repair_kernel(const ChunkScanArgs A, const int pop, const int32_t* __restri
         const int K = A.n_chunks[ind];
         const int sb = seg_base[ind];
         const int base = sym * A.n_seg + sb;
-        int2 prev = A.seg_out[base];
-        bool usable = A.seg_count[base] != 0xffffffffu;      // (a chunk that lost events to a full pool ends the walk: the lane is flagged later)
+        int2 prev = A.T.seg_out[base];
+        bool usable = A.T.seg_count[base] != SEG_LOST;      // (a chunk that lost events to a full pool ends the walk: the lane is flagged later)
         for (int c = 1; c < K && usable; ++c) {
-            const int2 a = A.seg_in[base + c];
+            const int2 a = A.T.seg_in[base + c];
             if (a.x != prev.x || a.y != prev.y) {
                 b200bt_chunk_item item;
                 item.individual = ind; item.chunk = c; item.segment = sb + c; item.n_chunks = K;
                 if (A.redo && lane == 0) A.redo[ind] = 1;
                 chunk_scan_item<VEC16, true>(A, item, sym, ws);      // (ends with a __syncwarp: its stores are visible to the warp)
             }
-            prev = A.seg_out[base + c];
-            usable = A.seg_count[base + c] != 0xffffffffu;
+            prev = A.T.seg_out[base + c];
+            usable = A.T.seg_count[base + c] != SEG_LOST;
         }
     }
 }
@@ -336,10 +357,10 @@ lane_repair_kernel(const ChunkScanArgs A, const int pop, const int32_t* __restri
 // ---- thread-per-lane scan ---------------------------------------------------------------------------
 // The warp-per-lane scan above spends a full warp on the scalar event chain of one lane.  With every lane cut
 // into the SAME K time chunks there are pop x S x K independent machines -- enough to give each one a THREAD:
-// a CTA owns (symbol, chunk, 256 individuals), streams tiles of the price row and the whole RSI bank of that
-// symbol through shared memory (cp.async, two stages) and every thread steps its own machine through the tile,
-// four bars per step.  The event path then runs in SIMT fashion for up to 32 lanes at once, all threads walk
-// the same bars (no tail), and the bank is fetched once per 256 lanes.  Events go to the same pool / segment
+// a warp takes (warp-slot, chunk, symbol) work items, stages tiles of the price row and of the (at most
+// LS_RSI_ROWS) RSI rows its 32 machines read through its own shared-memory ring (see "Tile movement"), and every
+// thread steps its own machine through the tile, four bars per step.  The event path then runs in SIMT fashion
+// for up to 32 lanes at once and all threads walk the same bars (no tail).  Events go to the same pool / segment
 // tables as the warp scan, so verification, repair and the metrics kernels are shared.
 #ifndef B200BT_LS_T
 #define B200BT_LS_T 128
@@ -395,14 +416,11 @@ struct LaneScanArgs {
     const float2* fine; int64_t n_fine;           // 4-bar ranges and their row stride
     int P, S; int64_t N;
     const b200bt_individual* indiv; const int32_t* slots; int n_slots; int pop; int K; int warm;
-    uint2* pool; int pool_blocks; int* next; unsigned* alloc;
-    int* seg_first; unsigned* seg_count; int2* seg_in; int2* seg_out; int* overflow;
+    SegTables T;
     unsigned* work;      // work-item counter of the persistent scan (zero at launch)
     int* stalls;         // [0] tiles that did not arrive in time (their items go to the exact fallback), [1..8] the first one's details
     long long wait_cycles;   // bound of a tile wait in SM clocks (LS_WAIT_CYCLES; b200bt_sweep_scan_wait_cycles overrides, for tests)
 };
-
-__device__ __forceinline__ int sym_of_block(unsigned bx, int S) { return (int)(bx % (unsigned)S); }
 
 // device-side tables the shared kernels expect: uniform K chunks per individual.  Work items are listed in dispatch
 // order (`order`: individuals by predicted cost, a lane's chunks adjacent), so that the 32 chunks a warp of the
@@ -453,10 +471,7 @@ __device__ __forceinline__ void lane_scan_give_up(const LaneScanArgs& A, const i
     const int k = wslot * 32 + (int)(threadIdx.x & 31);
     const int slot = k < A.n_slots ? (A.slots ? A.slots[k] : (k < A.pop ? k : -1)) : -1;
     if (slot < 0) return;
-    const int seg = sym * (A.pop * A.K) + slot * A.K + c;
-    A.seg_in[seg] = make_int2(0, -1);
-    A.seg_out[seg] = make_int2(0, -1);
-    A.seg_count[seg] = 0xffffffffu;
+    mark_lost(A.T, sym * (A.pop * A.K) + slot * A.K + c);
 }
 
 // -> false: a tile of this item did not arrive (see the wait below); the warp must not take another item
@@ -485,10 +500,8 @@ __device__ __forceinline__ bool lane_scan_item(const LaneScanArgs& A, const bool
     }
     __syncwarp();
     // The ring's barriers are initialised ONCE per warp (lane_scan_kernel) and their phases roll on from item to item: every
-    // copy of the previous item has landed and been waited for, so the ring continues at (ring_stage, ring_parity).  (The
-    // first persistent form invalidated and re-initialised the barriers at every item; about once in 10^4 launches a tile
-    // then never completed -- a re-initialisation racing with the copy engine's last update of the barrier it had just
-    // completed is the suspected cause -- which is also why the wait below is bounded.)
+    // copy of the previous item has landed and been waited for, so the ring continues at (ring_stage, ring_parity).
+    // (Invalidating and re-initialising them at every item lost a tile about once in 10^4 launches: DESIGN.md §3.1.)
 
     const int n = (int)A.N;
     const int T0 = (int)chunk_begin(A.N, c, A.K);       // first recorded bar (multiple of SW_GROUP, hence of LS_T)
@@ -509,11 +522,7 @@ __device__ __forceinline__ bool lane_scan_item(const LaneScanArgs& A, const bool
     const int my_row = 1 + __popc(heads & ((1u << leader) - 1u));       // staged row this machine reads
     if (n_rsi > LS_RSI_ROWS) {
         // not packed for this schedule: the lanes are flagged and re-run by the caller's exact fallback (fused kernel)
-        if (active) {
-            A.seg_in[seg] = make_int2(0, -1);
-            A.seg_out[seg] = make_int2(0, -1);
-            A.seg_count[seg] = 0xffffffffu;
-        }
+        if (active) mark_lost(A.T, seg);
         return true;
     }
     // lane L <= n_rsi issues the copies of staged row L (0 = price)
@@ -575,7 +584,16 @@ __device__ __forceinline__ bool lane_scan_item(const LaneScanArgs& A, const bool
     int cur_block = -1, fill = CK_BLOCK;
     unsigned count = 0;
     bool rec = false, dead = false;
-    uint2* wptr = A.pool;
+    uint2* wptr = A.T.pool;
+    auto record = [&](unsigned word, float p) {
+        if (fill == CK_BLOCK && !dead) {
+            const int b = pool_append(A.T, seg, cur_block);
+            if (b < 0) dead = true;
+            else { cur_block = b; fill = 0; wptr = A.T.pool + (int64_t)b * CK_BLOCK; }
+        }
+        if (!dead) { *wptr++ = make_uint2(word, __float_as_uint(p)); ++fill; }
+        ++count;
+    };
 
     // one bar of the state machine; same decisions as scan_window (sweep_dev.cuh).  Written as straight-line
     // selects: the threads of a warp that fire on the same bar (entries and exits alike) share one pass.
@@ -606,20 +624,7 @@ __device__ __forceinline__ bool lane_scan_item(const LaneScanArgs& A, const bool
         plo = flat ? p * mc[LS_THREADS] : -INFINITY;
         e_px = flat ? p : e_px;
         entry_bar = flat ? t : entry_bar;
-        if (rec) {
-            if (fill == CK_BLOCK && !dead) {
-                const int b = (int)atomicAdd(A.alloc, 1u);
-                if (b >= A.pool_blocks) { atomicExch(A.overflow, 1); dead = true; }
-                else {
-                    A.next[b] = -1;
-                    if (cur_block < 0) A.seg_first[seg] = b; else A.next[cur_block] = b;
-                    cur_block = b; fill = 0;
-                    wptr = A.pool + (int64_t)b * CK_BLOCK;
-                }
-            }
-            if (!dead) { *wptr++ = make_uint2(word, __float_as_uint(p)); ++fill; }
-            ++count;
-        }
+        if (rec) record(word, p);
     };
 
     int stage = ring_stage;
@@ -642,7 +647,7 @@ __device__ __forceinline__ bool lane_scan_item(const LaneScanArgs& A, const bool
         }
         const int t0 = (tl_begin + it) * LS_T;
         if (active) {
-            if (t0 == T0) { A.seg_in[seg] = make_int2(pos, pos != 0 ? entry_bar : -1); rec = true; }
+            if (t0 == T0) { A.T.seg_in[seg] = seg_state(pos, entry_bar); rec = true; }
             const float4* __restrict__ pp = reinterpret_cast<const float4*>(wtile + (size_t)stage * LS_ROWS * LS_STRIDE);
             const float4* __restrict__ rr = reinterpret_cast<const float4*>(wtile + ((size_t)stage * LS_ROWS + my_row) * LS_STRIDE);
             const float2* __restrict__ zp = wzone + (size_t)stage * LS_ROWS * ZR;
@@ -690,24 +695,10 @@ __device__ __forceinline__ bool lane_scan_item(const LaneScanArgs& A, const bool
     ring_stage = stage;
     ring_parity = parity;
     if (!active) return true;
-    A.seg_out[seg] = make_int2(pos, pos != 0 ? entry_bar : -1);
-    if (c == A.K - 1 && pos != 0)   // force-close at the last bar (:849-876)
-    {
-        rec = true;   // (the last chunk always records: T0 < N)
-        const unsigned word = (unsigned)(n - 1) | B200BT_EVENT_EXIT | (pos > 0 ? B200BT_EVENT_SELL : 0u);
-        if (fill == CK_BLOCK && !dead) {
-            const int b = (int)atomicAdd(A.alloc, 1u);
-            if (b >= A.pool_blocks) { atomicExch(A.overflow, 1); dead = true; }
-            else {
-                A.next[b] = -1;
-                if (cur_block < 0) A.seg_first[seg] = b; else A.next[cur_block] = b;
-                wptr = A.pool + (int64_t)b * CK_BLOCK;
-            }
-        }
-        if (!dead) *wptr = make_uint2(word, __float_as_uint(__ldg(A.price + (int64_t)sym * A.ld_price + (n - 1))));
-        ++count;
-    }
-    A.seg_count[seg] = dead ? 0xffffffffu : count;
+    A.T.seg_out[seg] = seg_state(pos, entry_bar);
+    if (c == A.K - 1 && pos != 0)   // force-close at the last bar (:849-876; the last chunk always records: T0 < N)
+        record((unsigned)(n - 1) | B200BT_EVENT_EXIT | (pos > 0 ? B200BT_EVENT_SELL : 0u), __ldg(A.price + (int64_t)sym * A.ld_price + (n - 1)));
+    A.T.seg_count[seg] = dead ? SEG_LOST : count;
     return true;
 }
 
@@ -773,12 +764,63 @@ struct ChunkPartial {
 };
 static_assert(sizeof(ChunkPartial) == 160, "ChunkPartial layout");
 
-// entry record a chunk's first exit is priced against, from the chunk's (verified) start state
-__device__ __forceinline__ void chunk_carry(const int2 in, const float* __restrict__ pr, unsigned& w_carry, float& p_carry) {
-    w_carry = 0u; p_carry = 0.f;
-    if (in.x != 0) {
-        w_carry = (unsigned)in.y | (in.x < 0 ? B200BT_EVENT_SELL : 0u);
-        p_carry = __ldg(pr + in.y);
+__device__ __forceinline__ unsigned seg_events(unsigned count) { return count == SEG_LOST ? 0u : count; }
+
+// One step of a chunk's records: records 2l and 2l+1 of the step in lane l (event word w, price pf), and the record
+// before 2l (lane l-1's second one; lane 0: the previous step's last record, or the entry the chunk starts in).
+struct RecordPair {
+    int cnt;                   // records in the step (1..64)
+    int last;                  // lane holding the step's last record
+    bool a0, a1;               // records 2l, 2l+1 exist
+    unsigned w0, w1, w_prev;
+    float pf0, pf1, p_prev;
+};
+
+// Cursor over the `count` records of segment `seg` in time order, 64 per step, two consecutive ones per lane (one 16-byte
+// load: half the shuffles per record):  for (RecordPair r; next_pair(R, r); advance(R, r)) { ... }.  A chain that leaves
+// the pool (a segment being re-scanned on the side stream) ends the walk.
+struct RecordReader {
+    const uint2* pool; const int* next; int pool_blocks;
+    unsigned left; int b, off;
+    unsigned w_carry; float p_carry;     // the record before the next step's first one
+};
+
+__device__ __forceinline__ RecordReader record_reader(const uint2* __restrict__ pool, const int* __restrict__ next, int pool_blocks,
+                                                      const int* __restrict__ seg_first, int seg, unsigned count, int2 in,
+                                                      const float* __restrict__ pr) {
+    RecordReader R{pool, next, pool_blocks, count, count ? seg_first[seg] : -1, 0, 0u, 0.f};
+    if (in.x != 0) {      // the entry record the chunk's first exit is priced against
+        R.w_carry = (unsigned)in.y | (in.x < 0 ? B200BT_EVENT_SELL : 0u);
+        R.p_carry = __ldg(pr + in.y);
+    }
+    if ((unsigned)R.b >= (unsigned)pool_blocks) R.left = 0;
+    return R;
+}
+
+__device__ __forceinline__ bool next_pair(const RecordReader& R, RecordPair& r) {
+    if (!R.left) return false;
+    const int lane = threadIdx.x & 31;
+    r.cnt = (int)min(64u, R.left);
+    r.last = (r.cnt - 1) >> 1;
+    r.a0 = 2 * lane < r.cnt; r.a1 = 2 * lane + 1 < r.cnt;
+    uint4 ev = make_uint4(0u, 0u, 0u, 0u);
+    if (r.a0) ev = *reinterpret_cast<const uint4*>(R.pool + (int64_t)R.b * CK_BLOCK + R.off + 2 * lane);   // (slot 2l+1 may be unused: in-block)
+    r.w0 = ev.x; r.w1 = ev.z;
+    r.pf0 = __uint_as_float(ev.y); r.pf1 = __uint_as_float(ev.w);
+    r.p_prev = __shfl_up_sync(FULL, r.pf1, 1);
+    r.w_prev = __shfl_up_sync(FULL, r.w1, 1);
+    if (lane == 0) { r.p_prev = R.p_carry; r.w_prev = R.w_carry; }
+    return true;
+}
+
+__device__ __forceinline__ void advance(RecordReader& R, const RecordPair& r) {
+    R.w_carry = __shfl_sync(FULL, (r.cnt & 1) ? r.w0 : r.w1, r.last);
+    R.p_carry = __shfl_sync(FULL, (r.cnt & 1) ? r.pf0 : r.pf1, r.last);
+    R.left -= r.cnt;
+    R.off += 64;
+    if (R.off == CK_BLOCK && R.left) {
+        R.b = R.next[R.b]; R.off = 0;
+        if ((unsigned)R.b >= (unsigned)R.pool_blocks) R.left = 0;
     }
 }
 
@@ -797,26 +839,13 @@ chunk_sums_kernel(const float* __restrict__ price, int64_t ld_price, const b200b
     const int seg = sym * n_seg + item.segment;
     const double size = indiv[item.individual].position_size;
     const double fee1 = __dmul_rn(size, 0.001), fee2 = __dmul_rn(size, 0.002);
-    unsigned left = seg_count[seg];
-    if (left == 0xffffffffu) left = 0;
-    unsigned w_carry; float p_carry;
-    chunk_carry(seg_in[seg], price + (int64_t)sym * ld_price, w_carry, p_carry);
-    int b = left ? seg_first[seg] : -1, off = 0;
-    if ((unsigned)b >= (unsigned)pool_blocks) left = 0;   // (a segment being re-scanned on the side stream)
     double run = 0.0, best = -INFINITY;
-    // 64 records per step, two consecutive ones per lane (one 16-byte load): half the shuffles per record
-    while (left) {
-        const int cnt = (int)min(64u, left);
-        const bool a0 = 2 * lane < cnt, a1 = 2 * lane + 1 < cnt;
-        uint4 ev = make_uint4(0u, 0u, 0u, 0u);
-        if (a0) ev = *reinterpret_cast<const uint4*>(pool + (int64_t)b * CK_BLOCK + off + 2 * lane);   // (slot 2l+1 may be unused: in-block)
-        const float pf0 = __uint_as_float(ev.y), pf1 = __uint_as_float(ev.w);
-        float p_prev = __shfl_up_sync(FULL, pf1, 1);
-        unsigned w_prev = __shfl_up_sync(FULL, ev.z, 1);
-        if (lane == 0) { p_prev = p_carry; w_prev = w_carry; }
+    RecordReader R = record_reader(pool, next, pool_blocks, seg_first, seg, seg_events(seg_count[seg]), seg_in[seg],
+                                   price + (int64_t)sym * ld_price);
+    for (RecordPair r; next_pair(R, r); advance(R, r)) {
         int dur;
-        const double pnl0 = record_pnl(a0, ev.x, pf0, w_prev, p_prev, size, fee1, fee2, dur);
-        const double pnl1 = record_pnl(a1, ev.z, pf1, ev.x, pf0, size, fee1, fee2, dur);
+        const double pnl0 = record_pnl(r.a0, r.w0, r.pf0, r.w_prev, r.p_prev, size, fee1, fee2, dur);
+        const double pnl1 = record_pnl(r.a1, r.w1, r.pf1, r.w0, r.pf0, size, fee1, fee2, dur);
         const double s2 = pnl0 + pnl1;
         double cs = s2;
 #pragma unroll
@@ -825,16 +854,8 @@ chunk_sums_kernel(const float* __restrict__ price, int64_t ld_price, const b200b
             if (lane >= d) cs += up;
         }
         const double after0 = run + (cs - s2) + pnl0, after1 = run + cs;
-        best = fmax(best, warp_max_d(fmax(a0 ? after0 : -INFINITY, a1 ? after1 : -INFINITY)));
+        best = fmax(best, warp_max_d(fmax(r.a0 ? after0 : -INFINITY, r.a1 ? after1 : -INFINITY)));
         run += shfl_d(cs, 31);
-        const int last = (cnt - 1) >> 1;
-        const unsigned wl = (cnt & 1) ? ev.x : ev.z;
-        const float pl = (cnt & 1) ? pf0 : pf1;
-        w_carry = __shfl_sync(FULL, wl, last);
-        p_carry = __shfl_sync(FULL, pl, last);
-        left -= cnt;
-        off += 64;
-        if (off == CK_BLOCK && left) { b = next[b]; off = 0; if ((unsigned)b >= (unsigned)pool_blocks) break; }
     }
     if (lane == 0) { seg_sum[seg] = run; seg_max[seg] = best; }
 }
@@ -867,8 +888,7 @@ chunk_partial_kernel(const float* __restrict__ price, int64_t ld_price, const b2
         const bool in = c < item.chunk;
         const double s = in ? seg_sum[base + c] : 0.0;
         const double mx = in ? seg_max[base + c] : -INFINITY;
-        unsigned n = in ? seg_count[base + c] : 0u;
-        if (n == 0xffffffffu) n = 0;
+        const unsigned n = in ? seg_events(seg_count[base + c]) : 0u;
         double incl = s;
 #pragma unroll
         for (int d = 1; d < 32; d <<= 1) {
@@ -906,26 +926,15 @@ chunk_partial_kernel(const float* __restrict__ price, int64_t ld_price, const b2
         else day_complete(da, x);
     };
 
-    unsigned left = seg_count[seg];
-    if (left == 0xffffffffu) left = 0;
-    const unsigned count = left;
-    unsigned w_carry; float p_carry;
-    chunk_carry(seg_in[seg], price + (int64_t)sym * ld_price, w_carry, p_carry);
-    int b = left ? seg_first[seg] : -1, off = 0;
-    if ((unsigned)b >= (unsigned)pool_blocks) left = 0;
-    // 64 records per step, two consecutive ones per lane (record 2l and 2l+1 of the step: one 16-byte load)
-    while (left) {
-        const int cnt = (int)min(64u, left);
-        const bool a0 = 2 * lane < cnt, a1 = 2 * lane + 1 < cnt;
-        uint4 ev = make_uint4(0u, 0u, 0u, 0u);
-        if (a0) ev = *reinterpret_cast<const uint4*>(pool + (int64_t)b * CK_BLOCK + off + 2 * lane);
-        const unsigned w0 = ev.x, w1 = ev.z;
-        const float pf0 = __uint_as_float(ev.y), pf1 = __uint_as_float(ev.w);
-        float p_prev = __shfl_up_sync(FULL, pf1, 1);
-        unsigned w_prev = __shfl_up_sync(FULL, w1, 1);
-        if (lane == 0) { p_prev = p_carry; w_prev = w_carry; }
+    const unsigned count = seg_events(seg_count[seg]);
+    RecordReader R = record_reader(pool, next, pool_blocks, seg_first, seg, count, seg_in[seg], price + (int64_t)sym * ld_price);
+    for (RecordPair r; next_pair(R, r); advance(R, r)) {
+        const int cnt = r.cnt, last_lane = r.last;
+        const bool a0 = r.a0, a1 = r.a1;
+        const unsigned w0 = r.w0, w1 = r.w1;
+        const float pf0 = r.pf0, pf1 = r.pf1;
         int dur0, dur1;
-        const double pnl0 = record_pnl(a0, w0, pf0, w_prev, p_prev, size, fee1, fee2, dur0);
+        const double pnl0 = record_pnl(a0, w0, pf0, r.w_prev, r.p_prev, size, fee1, fee2, dur0);
         const double pnl1 = record_pnl(a1, w1, pf1, w0, pf0, size, fee1, fee2, dur1);
         if (pnl0 > 0.0) { l_gain += pnl0; ++l_win; l_maxp = fmax(l_maxp, pnl0); }
         else if (pnl0 < 0.0) { l_loss += pnl0; ++l_los; l_minl = fmin(l_minl, pnl0); }
@@ -977,7 +986,6 @@ chunk_partial_kernel(const float* __restrict__ price, int64_t ld_price, const b2
         equity += batch_sum;
 
         // calendar-day buckets
-        const int last_lane = (cnt - 1) >> 1;
         const int d0 = a0 ? day_of(w0) : 0;
         const int d1 = a1 ? day_of(w1) : d0;
         const int first_day = __shfl_sync(FULL, d0, 0);
@@ -1025,11 +1033,6 @@ chunk_partial_kernel(const float* __restrict__ price, int64_t ld_price, const b2
         day_valid = 1;
 
         index += cnt;
-        w_carry = __shfl_sync(FULL, (cnt & 1) ? w0 : w1, last_lane);
-        p_carry = __shfl_sync(FULL, (cnt & 1) ? pf0 : pf1, last_lane);
-        left -= cnt;
-        off += 64;
-        if (off == CK_BLOCK && left) { b = next[b]; off = 0; if ((unsigned)b >= (unsigned)pool_blocks) break; }
     }
     // per-lane accumulators -> chunk totals
     const double tot_profit = warp_sum_d(l_gain), tot_loss = warp_sum_d(l_loss);
@@ -1095,7 +1098,7 @@ __global__ void lane_combine_kernel(const b200bt_individual* __restrict__ indiv,
             const int2 z = seg_out[base + c - 1];
             ok = ok && (a.x == z.x) && (a.y == z.y);
         }
-        ok = ok && (seg_count[base + c] != 0xffffffffu);
+        ok = ok && (seg_count[base + c] != SEG_LOST);
     }
     invalid[t] = ok ? 0 : 1;
     if (!ok) return;
@@ -1159,43 +1162,73 @@ using namespace b200bt;
 
 namespace {
 
-constexpr int REPAIR_COUNTERS = 130;   // work counters: [0] bounded repair pass, [1] overlapped pass, [last] the scan; 2 + REPAIR_COUNTERS a multiple of 4 (alignment)
+// Counters of one sweep, zeroed with the segment tables at entry.  The first four words are what the caller's
+// overflow_host_or_null[0..3] receives.
+struct SweepCounters {
+    int overflow;              // [0] the event pool ran out of blocks
+    int n_flagged;             // [1] (individual, symbol) lanes that went through the exact fallback
+    unsigned alloc;            // [2] pool blocks handed out
+    int scan_stalls[9];        // [3] tiles of lane_scan_kernel that did not arrive in time; [1..8] the first one's details
+    unsigned repair_work[2];   // work counters of chunk_repair_kernel and lane_repair_kernel
+    unsigned scan_work;        // work counter of lane_scan_kernel
+    int n_fix, n_redo;         // items in fix_items, individuals in redo_list
+};
+static_assert(offsetof(SweepCounters, scan_stalls) == 3 * sizeof(int), "host flags: the first four words");
+
+// Workspace of the time-chunked sweeps.  Every region starts 16-byte aligned (the base must be); the segment tables
+// and the counters follow one another, so one memset clears them.
 struct ChunkWorkspace {
-    uint2* pool; int2* seg_in; int2* seg_out; int* seg_first; unsigned* seg_count; unsigned* alloc; int* overflow;
-    unsigned* n_repair; int4* repair; int* next; ChunkPartial* partial; double* seg_sum; double* seg_max;
-    b200bt_chunk_item* fix_items; int* n_fix; unsigned char* redo;   // overlapped repair tail (n_seg items, pop flags)
-    unsigned char* end;
+    SegTables T;                           // pool, next [pool_blocks] (apart); seg_* [segs]; alloc, overflow -> ctr
+    SweepCounters* ctr;
+    ChunkPartial* partial;                 // [segs]
+    double* seg_sum; double* seg_max;      // [segs] PnL sum and largest prefix sum of the chunk's records
+    b200bt_chunk_item* fix_items;          // [n_seg] chunks of the individuals lane_repair_kernel touched; once their
+    int32_t* redo_list;                    // metrics are recomputed the same memory holds [pop] individuals to re-run
+    unsigned char* redo;                   // [pop] individuals lane_repair_kernel touched
+    b200bt_chunk_item* items; int32_t* seg_base; int32_t* n_chunks;   // b200bt_sweep_tiled: lane tables [n_seg], [pop], [pop]
+    int64_t bytes;                         // end of the last region
+    size_t cleared;                        // bytes from seg_in to the end of the counters: they start at zero
 };
 
-// pool[pool_blocks][256] uint2 | seg_in[segs] int2 | seg_out[segs] int2 | seg_first[segs] | seg_count[segs] |
-// alloc, overflow, n_repair[REPAIR_COUNTERS] (work counters) | repair[segs] int4 (reserved) | next[pool_blocks] | (16-byte aligned) partial[segs] (128 B) |
-// seg_sum[segs] | seg_max[segs] | fix_items[n_seg] (16 B) | n_fix (16 B) | redo[pop]
-// (wide types first: the base must be 16-byte aligned)
-ChunkWorkspace carve(void* workspace, int pool_blocks, int64_t segs, int n_seg, int pop) {
-    ChunkWorkspace w;
-    w.pool = (uint2*)workspace;
-    w.seg_in = (int2*)(w.pool + (int64_t)pool_blocks * CK_BLOCK);
-    w.seg_out = w.seg_in + segs;
-    w.seg_first = (int*)(w.seg_out + segs);
-    w.seg_count = (unsigned*)(w.seg_first + segs);
-    w.alloc = w.seg_count + segs;
-    w.overflow = (int*)(w.alloc + 1);
-    w.n_repair = (unsigned*)(w.overflow + 1);
-    w.repair = (int4*)(((uintptr_t)(w.n_repair + REPAIR_COUNTERS) + 15) & ~(uintptr_t)15);
-    w.next = (int*)(w.repair + segs);
-    w.partial = (ChunkPartial*)(((uintptr_t)(w.next + pool_blocks) + 15) & ~(uintptr_t)15);
-    w.seg_sum = (double*)(w.partial + segs);
-    w.seg_max = w.seg_sum + segs;
-    w.fix_items = (b200bt_chunk_item*)(w.seg_max + segs);
-    w.n_fix = (int*)(w.fix_items + n_seg);
-    w.redo = (unsigned char*)(w.n_fix + 4);
-    w.end = w.redo + ((pop + 15) & ~15);
+template <class T>
+void take(uintptr_t& at, T*& p, int64_t n) {
+    at = (at + 15) & ~(uintptr_t)15;
+    p = reinterpret_cast<T*>(at);
+    at += (uintptr_t)n * sizeof(T);
+}
+
+// Lays the workspace out from `base` (nullptr: only `bytes` is wanted).  `tiled` adds the lane tables.
+ChunkWorkspace carve(void* base, int pool_blocks, int64_t segs, int n_seg, int pop, bool tiled) {
+    ChunkWorkspace w{};
+    uintptr_t at = (uintptr_t)base;
+    take(at, w.T.pool, (int64_t)pool_blocks * CK_BLOCK);
+    take(at, w.T.seg_in, segs); take(at, w.T.seg_out, segs); take(at, w.T.seg_first, segs); take(at, w.T.seg_count, segs);
+    take(at, w.ctr, 1);
+    take(at, w.T.next, pool_blocks);
+    take(at, w.partial, segs); take(at, w.seg_sum, segs); take(at, w.seg_max, segs);
+    take(at, w.fix_items, n_seg);
+    w.redo_list = reinterpret_cast<int32_t*>(w.fix_items);     // (pop <= n_seg)
+    take(at, w.redo, pop);
+    if (tiled) { take(at, w.items, n_seg); take(at, w.seg_base, pop); take(at, w.n_chunks, pop); }
+    w.bytes = (int64_t)(at - (uintptr_t)base);
+    w.cleared = (size_t)((char*)(w.ctr + 1) - (char*)w.T.seg_in);
+    w.T.pool_blocks = pool_blocks; w.T.alloc = &w.ctr->alloc; w.T.overflow = &w.ctr->overflow;
     return w;
 }
 
-int64_t chunk_workspace_bytes(int pool_blocks, int64_t segs, int n_seg, int pop) {
-    return (int64_t)pool_blocks * CK_BLOCK * 8 + segs * 16 + (segs * 2 + 2 + REPAIR_COUNTERS) * 4 + 16 + segs * 16 + (int64_t)pool_blocks * 4 + 16 +
-           segs * (int64_t)(sizeof(ChunkPartial) + 16) + (int64_t)n_seg * 16 + 16 + ((pop + 15) & ~15);
+// rows the scan kernels may copy 16 bytes at a time
+bool rows_vec16(const float* price, int64_t ld_price, const float* rsi, int64_t ld_rsi) {
+    return (((uintptr_t)price | (uintptr_t)rsi) & 15) == 0 && ld_price % 4 == 0 && ld_rsi % 4 == 0;
+}
+
+ChunkScanArgs chunk_scan_args(const float* price, int64_t ld_price, const float* rsi, int64_t ld_rsi, int P, int S, int64_t N,
+                              const b200bt_individual* indiv, const b200bt_chunk_item* items, int n_items, int n_seg, int warm,
+                              const int32_t* n_chunks, const ChunkWorkspace& w) {
+    ChunkScanArgs A;
+    A.price = price; A.ld_price = ld_price; A.rsi = rsi; A.ld_rsi = ld_rsi; A.P = P; A.S = S; A.N = N;
+    A.indiv = indiv; A.items = items; A.n_items = n_items; A.n_seg = n_seg; A.warm = warm;
+    A.T = w.T; A.n_chunks = n_chunks; A.redo = nullptr;
+    return A;
 }
 
 // second stream + events for the overlapped repair tail, one set per device
@@ -1219,29 +1252,17 @@ int side_stream(SideStream** out) {
     return B200BT_OK;
 }
 
-// the bounded repair pass on the critical path can be switched off (B200BT_MAIN_REPAIR=0: everything in the overlapped pass)
-int main_repair_rounds() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("B200BT_MAIN_REPAIR");
-        v = e ? atoi(e) : 1;
-    }
-    return v;
-}
-
-// Everything after the speculative scan: verify + repair (lane_repair_kernel) -> chunk-parallel metrics.
+// Everything after the speculative scan: verify + repair -> chunk-parallel metrics.
 //
 // chunk_repair_kernel on the critical path makes almost every lane consistent; what it leaves is a handful of lanes whose
 // trajectories do not meet the recorded ones inside a chunk (always in the market) and which have to be re-scanned chunk
 // after chunk by a single warp each.  That is lane_repair_kernel, on another stream BESIDE the metrics kernels of all
 // lanes; the individuals it touches are flagged and only their metrics are recomputed afterwards.
 // max_repair_rounds: 0 = no repair (every inconsistent lane takes the exact fallback), 1 = chunk_repair_kernel only, >= 2 = both.
-int finish_chunks(const ChunkScanArgs& A, const ChunkWorkspace& w, const b200bt_chunk_item* items, int n_items,
-                  const int32_t* seg_base, int pop, int max_repair_rounds, const b200bt_sweep_config* cfg_host,
-                  b200bt_lane_stats* stats, uint32_t* events, int64_t event_cap, unsigned char* lane_invalid,
-                  int* overflow_host_or_null, cudaStream_t st) {
-    const int S = A.S, n_seg = A.n_seg;
-    const bool vec16 = (((uintptr_t)A.price | (uintptr_t)A.rsi) & 15) == 0 && A.ld_price % 4 == 0 && A.ld_rsi % 4 == 0;
+int finish_chunks(const ChunkScanArgs& A, const ChunkWorkspace& w, const bool vec16, const int32_t* seg_base, int pop,
+                  int max_repair_rounds, const b200bt_sweep_config* cfg_host, b200bt_lane_stats* stats, uint32_t* events,
+                  int64_t event_cap, unsigned char* lane_invalid, int* overflow_host_or_null, cudaStream_t st) {
+    const int S = A.S, n_seg = A.n_seg, n_items = A.n_items;
     auto kern_fix = vec16 ? chunk_repair_kernel<true> : chunk_repair_kernel<false>;
     auto kern_walk = vec16 ? lane_repair_kernel<true> : lane_repair_kernel<false>;
     const size_t smem = sizeof(WarpShared) * SW_WARPS;
@@ -1253,78 +1274,70 @@ int finish_chunks(const ChunkScanArgs& A, const ChunkWorkspace& w, const b200bt_
     B200BT_REQUIRE(mblocks < (1ll << 31), B200BT_ELIMIT, "sweep_chunked: too many work items");
     B200BT_REQUIRE(lanes < (1ll << 30), B200BT_ELIMIT, "sweep_chunked: too many lanes");
 
-    // Both repair kernels run a persistent grid (3 CTAs per SM) whose warps take work from a counter (n_repair[0], [1]).
+    // Both repair kernels run a persistent grid (3 CTAs per SM) whose warps take work from a counter (repair_work).
     int dev = 0, sms = 148;
     if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     const unsigned repair_grid = 3u * (unsigned)sms;
-    auto repair_pass = [&](cudaStream_t rs, int pass, unsigned char* redo) -> int {
-        ChunkScanArgs R = A;
-        R.redo = redo;
-        if (pass == 0) kern_fix<<<repair_grid, SW_WARPS * 32, smem, rs>>>(R, w.n_repair);
-        else kern_walk<<<repair_grid, SW_WARPS * 32, smem, rs>>>(R, pop, seg_base, w.n_repair + 1);
-        B200BT_LAUNCH_CHECK("repair launch");
-        return B200BT_OK;
-    };
     // (the fix-up pass reuses the full-size grid with a device-side item count: CTAs beyond it leave at once)
     auto metrics = [&](const b200bt_chunk_item* its, const int* n_dev) -> int {
-        chunk_sums_kernel<<<(unsigned)mblocks, 128, 0, st>>>(A.price, A.ld_price, A.indiv, its, n_items, S, n_seg, w.pool, w.next,
-                                                              w.seg_first, w.seg_count, w.seg_in, w.seg_sum, w.seg_max, n_dev, A.pool_blocks);
+        chunk_sums_kernel<<<(unsigned)mblocks, 128, 0, st>>>(A.price, A.ld_price, A.indiv, its, n_items, S, n_seg, w.T.pool, w.T.next,
+                                                              w.T.seg_first, w.T.seg_count, w.T.seg_in, w.seg_sum, w.seg_max, n_dev,
+                                                              w.T.pool_blocks);
         B200BT_LAUNCH_CHECK("chunk_sums launch");
-        chunk_partial_kernel<<<(unsigned)mblocks, 128, 0, st>>>(A.price, A.ld_price, A.indiv, its, n_items, S, n_seg, w.pool, w.next,
-                                                                 w.seg_first, w.seg_count, w.seg_in, w.seg_sum, w.seg_max,
-                                                                 *cfg_host, events, event_cap, w.partial, n_dev, A.pool_blocks);
+        chunk_partial_kernel<<<(unsigned)mblocks, 128, 0, st>>>(A.price, A.ld_price, A.indiv, its, n_items, S, n_seg, w.T.pool, w.T.next,
+                                                                 w.T.seg_first, w.T.seg_count, w.T.seg_in, w.seg_sum, w.seg_max,
+                                                                 *cfg_host, events, event_cap, w.partial, n_dev, w.T.pool_blocks);
         B200BT_LAUNCH_CHECK("chunk_partial launch");
         return B200BT_OK;
     };
 
     int rc = B200BT_OK;
-    const bool main_pass = max_repair_rounds >= 1 && main_repair_rounds() != 0;
-    const bool tail = max_repair_rounds >= 2 || (max_repair_rounds >= 1 && !main_pass);
-    if (main_pass && (rc = repair_pass(st, 0, nullptr))) return rc;
+    const bool tail = max_repair_rounds >= 2;
+    if (max_repair_rounds >= 1) {
+        kern_fix<<<repair_grid, SW_WARPS * 32, smem, st>>>(A, &w.ctr->repair_work[0]);
+        B200BT_LAUNCH_CHECK("repair launch");
+    }
     SideStream* side = nullptr;
-    e = cudaMemsetAsync(w.n_fix, 0, 16 + ((pop + 15) & ~15), st);   // n_fix, redo-list length, flagged lanes + redo flags
+    e = cudaMemsetAsync(w.redo, 0, (size_t)pop, st);
     if (e != cudaSuccess) return cuda_status(e, "sweep_chunked: memset");
     if (tail) {
         if ((rc = side_stream(&side))) return rc;
         e = cudaEventRecord(side->fork, st);
         if (e != cudaSuccess) return cuda_status(e, "sweep_chunked: fork");
     }
-    if ((rc = metrics(items, nullptr))) return rc;
+    if ((rc = metrics(A.items, nullptr))) return rc;
     if (tail) {
         e = cudaStreamWaitEvent(side->stream, side->fork, 0);
         if (e != cudaSuccess) return cuda_status(e, "sweep_chunked: side wait");
-        if ((rc = repair_pass(side->stream, 1, w.redo))) return rc;
+        ChunkScanArgs R = A;
+        R.redo = w.redo;
+        kern_walk<<<repair_grid, SW_WARPS * 32, smem, side->stream>>>(R, pop, seg_base, &w.ctr->repair_work[1]);
+        B200BT_LAUNCH_CHECK("repair launch");
         e = cudaEventRecord(side->join, side->stream);
         if (e == cudaSuccess) e = cudaStreamWaitEvent(st, side->join, 0);
         if (e != cudaSuccess) return cuda_status(e, "sweep_chunked: join");
-        fix_items_kernel<<<(n_items + 255) / 256, 256, 0, st>>>(items, n_items, w.redo, w.fix_items, w.n_fix);
+        fix_items_kernel<<<(n_items + 255) / 256, 256, 0, st>>>(A.items, n_items, w.redo, w.fix_items, &w.ctr->n_fix);
         B200BT_LAUNCH_CHECK("fix_items launch");
-        if ((rc = metrics(w.fix_items, w.n_fix))) return rc;
+        if ((rc = metrics(w.fix_items, &w.ctr->n_fix))) return rc;
     }
-    lane_combine_kernel<<<(unsigned)((lanes + 127) / 128), 128, 0, st>>>(A.indiv, pop, S, seg_base, A.n_chunks, n_seg, w.seg_count,
-                                                                        w.seg_in, w.seg_out, w.partial, *cfg_host, stats,
+    lane_combine_kernel<<<(unsigned)((lanes + 127) / 128), 128, 0, st>>>(A.indiv, pop, S, seg_base, A.n_chunks, n_seg, w.T.seg_count,
+                                                                        w.T.seg_in, w.T.seg_out, w.partial, *cfg_host, stats,
                                                                         lane_invalid);
     B200BT_LAUNCH_CHECK("lane_combine launch");
     // exact fallback, driven from the device: the flagged individuals are listed and re-evaluated by the fused (serial)
-    // kernel; with nothing flagged its warps leave at once.  [n_fix + 1] = list length, [n_fix + 2] = flagged lanes.
-    int32_t* redo_list = reinterpret_cast<int32_t*>(w.fix_items);      // (the fix-up item list is no longer needed)
-    redo_list_kernel<<<(pop + 127) / 128, 128, 0, st>>>(pop, S, lane_invalid, redo_list, w.n_fix + 1, w.n_fix + 2);
+    // kernel; with nothing flagged its warps leave at once
+    redo_list_kernel<<<(pop + 127) / 128, 128, 0, st>>>(pop, S, lane_invalid, w.redo_list, &w.ctr->n_redo, &w.ctr->n_flagged);
     B200BT_LAUNCH_CHECK("redo_list launch");
-    if ((rc = launch_sweep(A.price, A.ld_price, A.rsi, A.ld_rsi, A.P, S, A.N, A.indiv, redo_list, pop, w.n_fix + 1, cfg_host, stats,
-                           events, event_cap, st)))
+    if ((rc = launch_sweep(A.price, A.ld_price, A.rsi, A.ld_rsi, A.P, S, A.N, A.indiv, w.redo_list, pop, &w.ctr->n_redo, cfg_host,
+                           stats, events, event_cap, st)))
         return rc;
-    if (overflow_host_or_null) {
-        // [0] = the event pool overflowed, [1] = lanes that went through the fallback, [2] = pool blocks handed out, [3] = tiles
-        // of the thread-per-lane scan that did not arrive in time (read by the host after its next sync)
-        e = cudaMemcpyAsync(overflow_host_or_null, w.overflow, sizeof(int), cudaMemcpyDeviceToHost, st);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(overflow_host_or_null + 1, w.n_fix + 2, sizeof(int), cudaMemcpyDeviceToHost, st);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(overflow_host_or_null + 2, w.alloc, sizeof(int), cudaMemcpyDeviceToHost, st);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(overflow_host_or_null + 3, w.n_repair + 64, sizeof(int), cudaMemcpyDeviceToHost, st);
+    if (overflow_host_or_null) {      // (read by the host after its next sync)
+        e = cudaMemcpyAsync(overflow_host_or_null, w.ctr, 4 * sizeof(int), cudaMemcpyDeviceToHost, st);
         if (e != cudaSuccess) return cuda_status(e, "sweep_chunked: overflow readback");
     }
     if (trace_launches()) {
         int d[9];
-        if (cudaMemcpy(d, w.n_repair + 64, sizeof(d), cudaMemcpyDeviceToHost) == cudaSuccess && d[0])
+        if (cudaMemcpy(d, w.ctr->scan_stalls, sizeof(d), cudaMemcpyDeviceToHost) == cudaSuccess && d[0])
             fprintf(stderr, "[b200bt] lane_scan: %d tile(s) timed out; first: block %d warp %d item(wslot,sym,c) %d,%d,%d tile %d of %d stage %d parity %d tl_begin %d rows %d\n",
                     d[0], d[1], d[2], d[3] >> 16, (d[3] >> 8) & 255, d[3] & 255, d[4], d[5], d[6] >> 1, d[6] & 1, d[7], d[8]);
     }
@@ -1347,7 +1360,7 @@ int check_sweep_args(const char* who, const float* price, int64_t ld_price, cons
 }  // namespace
 
 extern "C" int64_t b200bt_sweep_chunked_workspace_bytes(int pool_blocks, int S, int n_seg) {
-    return chunk_workspace_bytes(pool_blocks, (int64_t)S * n_seg, n_seg, n_seg);   // pop <= n_seg
+    return carve(nullptr, pool_blocks, (int64_t)S * n_seg, n_seg, n_seg, false).bytes;   // pop <= n_seg
 }
 
 extern "C" int b200bt_sweep_chunked(const float* price, int64_t ld_price, const float* rsi, int64_t ld_rsi, int P, int S,
@@ -1371,17 +1384,12 @@ extern "C" int b200bt_sweep_chunked(const float* price, int64_t ld_price, const 
     cudaStream_t st = (cudaStream_t)stream;
     const int64_t segs = (int64_t)S * n_seg;
     B200BT_REQUIRE(pop <= n_seg, B200BT_EINVAL, "sweep_chunked: fewer segments than individuals");
-    const ChunkWorkspace w = carve(workspace, pool_blocks, segs, n_seg, pop);
-    cudaError_t e = cudaMemsetAsync(w.seg_in, 0, (size_t)(segs * 6 + 2 + REPAIR_COUNTERS) * 4, st);
+    const ChunkWorkspace w = carve(workspace, pool_blocks, segs, n_seg, pop, false);
+    cudaError_t e = cudaMemsetAsync(w.T.seg_in, 0, w.cleared, st);
     if (e != cudaSuccess) return cuda_status(e, "sweep_chunked: memset");
 
-    ChunkScanArgs A;
-    A.price = price; A.ld_price = ld_price; A.rsi = rsi; A.ld_rsi = ld_rsi; A.P = P; A.S = S; A.N = N;
-    A.indiv = indiv; A.items = items; A.n_items = n_items; A.n_seg = n_seg; A.warm = warm;
-    A.pool = w.pool; A.pool_blocks = pool_blocks; A.next = w.next; A.alloc = w.alloc;
-    A.seg_first = w.seg_first; A.seg_count = w.seg_count; A.seg_in = w.seg_in; A.seg_out = w.seg_out; A.overflow = w.overflow;
-    A.n_chunks = n_chunks; A.redo = nullptr;
-    const bool vec16 = (((uintptr_t)price | (uintptr_t)rsi) & 15) == 0 && ld_price % 4 == 0 && ld_rsi % 4 == 0;
+    const ChunkScanArgs A = chunk_scan_args(price, ld_price, rsi, ld_rsi, P, S, N, indiv, items, n_items, n_seg, warm, n_chunks, w);
+    const bool vec16 = rows_vec16(price, ld_price, rsi, ld_rsi);
     auto kern = vec16 ? chunk_scan_kernel<true> : chunk_scan_kernel<false>;
     const size_t smem = sizeof(WarpShared) * SW_WARPS;
     e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -1390,8 +1398,8 @@ extern "C" int b200bt_sweep_chunked(const float* price, int64_t ld_price, const 
     B200BT_REQUIRE(blocks < (1ll << 31), B200BT_ELIMIT, "sweep_chunked: too many work items");
     kern<<<(unsigned)blocks, SW_WARPS * 32, smem, st>>>(A);
     B200BT_LAUNCH_CHECK("chunk_scan launch");
-    return finish_chunks(A, w, items, n_items, seg_base, pop, max_repair_rounds, cfg_host, stats, events, event_cap,
-                         lane_invalid, overflow_host_or_null, st);
+    return finish_chunks(A, w, vec16, seg_base, pop, max_repair_rounds, cfg_host, stats, events, event_cap, lane_invalid,
+                         overflow_host_or_null, st);
 }
 
 extern "C" int64_t b200bt_zone_map_floats(int P, int S, int64_t N) {
@@ -1419,7 +1427,7 @@ extern "C" int b200bt_zone_map(const float* price, int64_t ld_price, const float
 
 extern "C" int64_t b200bt_sweep_tiled_workspace_bytes(int pool_blocks, int S, int pop, int K) {
     const int64_t n_seg = (int64_t)pop * K;
-    return chunk_workspace_bytes(pool_blocks, S * n_seg, (int)n_seg, pop) + 16 + n_seg * 16 + (int64_t)pop * 8;
+    return carve(nullptr, pool_blocks, S * n_seg, (int)n_seg, pop, true).bytes;
 }
 
 // measurement hook: a pair of caller-owned CUDA events recorded around the scan kernel of the next b200bt_sweep_tiled calls
@@ -1460,13 +1468,10 @@ extern "C" int b200bt_sweep_tiled(const float* price, int64_t ld_price, const fl
     cudaStream_t st = (cudaStream_t)stream;
     const int n_seg = pop * K;
     const int64_t segs = (int64_t)S * n_seg;
-    const ChunkWorkspace w = carve(workspace, pool_blocks, segs, n_seg, pop);
-    b200bt_chunk_item* items = (b200bt_chunk_item*)(((uintptr_t)w.end + 15) & ~(uintptr_t)15);
-    int32_t* seg_base = (int32_t*)(items + n_seg);
-    int32_t* n_chunks = seg_base + pop;
-    cudaError_t e = cudaMemsetAsync(w.seg_in, 0, (size_t)(segs * 6 + 2 + REPAIR_COUNTERS) * 4, st);
+    const ChunkWorkspace w = carve(workspace, pool_blocks, segs, n_seg, pop, true);
+    cudaError_t e = cudaMemsetAsync(w.T.seg_in, 0, w.cleared, st);
     if (e != cudaSuccess) return cuda_status(e, "sweep_tiled: memset");
-    lane_tables_kernel<<<(n_seg + 255) / 256, 256, 0, st>>>(pop, K, order, items, seg_base, n_chunks);
+    lane_tables_kernel<<<(n_seg + 255) / 256, 256, 0, st>>>(pop, K, order, w.items, w.seg_base, w.n_chunks);
     B200BT_LAUNCH_CHECK("lane_tables launch");
 
     LaneScanArgs L;
@@ -1474,18 +1479,17 @@ extern "C" int b200bt_sweep_tiled(const float* price, int64_t ld_price, const fl
     L.zones = (const float2*)zones_or_null; L.n_zone_blocks = zone_row_stride(N);    // (row stride of the zone map)
     L.fine = zones_or_null ? L.zones + (int64_t)S * (P + 1) * zone_row_stride(N) : nullptr; L.n_fine = zone_fine_stride(N);
     L.indiv = indiv; L.slots = slots; L.n_slots = n_slots; L.pop = pop; L.K = K; L.warm = warm;
-    L.pool = w.pool; L.pool_blocks = pool_blocks; L.next = w.next; L.alloc = w.alloc;
-    L.seg_first = w.seg_first; L.seg_count = w.seg_count; L.seg_in = w.seg_in; L.seg_out = w.seg_out; L.overflow = w.overflow;
-    const bool vec16 = (((uintptr_t)price | (uintptr_t)rsi) & 15) == 0 && ld_price % 4 == 0 && ld_rsi % 4 == 0;
+    L.T = w.T;
+    L.work = &w.ctr->scan_work;
+    L.stalls = w.ctr->scan_stalls;
+    L.wait_cycles = g_wait_cycles != 0 ? g_wait_cycles : LS_WAIT_CYCLES;
+    const bool vec16 = rows_vec16(price, ld_price, rsi, ld_rsi);
     auto kern = zones_or_null ? lane_scan_kernel<true> : lane_scan_kernel<false>;
     e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
     if (e != cudaSuccess) return cuda_status(e, "sweep_tiled: cudaFuncSetAttribute");
     const int64_t n_items = (int64_t)(n_slots / 32) * K * S;
     B200BT_REQUIRE(n_items < (1ll << 30), B200BT_ELIMIT, "sweep_tiled: too many work items");
-    L.work = w.n_repair + REPAIR_COUNTERS - 1;      // (a counter no repair round uses; zeroed with the rest above)
-    L.stalls = reinterpret_cast<int*>(w.n_repair + 64);   // (counters 64..72, zeroed with the rest)
-    L.wait_cycles = g_wait_cycles != 0 ? g_wait_cycles : LS_WAIT_CYCLES;
     // persistent grid: one resident set of CTAs (warps take work items from the counter), no more CTAs than items need
     int dev = 0, sms = 0, per_sm = 0;
     e = cudaGetDevice(&dev);
@@ -1499,12 +1503,7 @@ extern "C" int b200bt_sweep_tiled(const float* price, int64_t ld_price, const fl
     if (g_scan_ev[1]) cudaEventRecord(g_scan_ev[1], st);
     B200BT_LAUNCH_CHECK("lane_scan launch");
 
-    ChunkScanArgs A;   // for the shared repair / metrics kernels
-    A.price = price; A.ld_price = ld_price; A.rsi = rsi; A.ld_rsi = ld_rsi; A.P = P; A.S = S; A.N = N;
-    A.indiv = indiv; A.items = items; A.n_items = n_seg; A.n_seg = n_seg; A.warm = warm;
-    A.pool = w.pool; A.pool_blocks = pool_blocks; A.next = w.next; A.alloc = w.alloc;
-    A.seg_first = w.seg_first; A.seg_count = w.seg_count; A.seg_in = w.seg_in; A.seg_out = w.seg_out; A.overflow = w.overflow;
-    A.n_chunks = n_chunks; A.redo = nullptr;
-    return finish_chunks(A, w, items, n_seg, seg_base, pop, max_repair_rounds, cfg_host, stats, events, event_cap, lane_invalid,
+    const ChunkScanArgs A = chunk_scan_args(price, ld_price, rsi, ld_rsi, P, S, N, indiv, w.items, n_seg, n_seg, warm, w.n_chunks, w);
+    return finish_chunks(A, w, vec16, w.seg_base, pop, max_repair_rounds, cfg_host, stats, events, event_cap, lane_invalid,
                          overflow_host_or_null, st);
 }

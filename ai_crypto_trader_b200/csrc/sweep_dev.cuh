@@ -51,10 +51,6 @@ struct WarpAcc {
     uint32_t* ev_out;
     unsigned n_win, n_loss, n_days, n_events;
     int day_valid, pivot_set;
-    // chunk-parallel metrics only: the first calendar day of a chunk may continue the previous chunk's
-    // last day, so its sum is kept aside instead of being counted as a finished day
-    int hold_first, first_done, first_day;
-    double first_sum;
     double npivot, ns1, ns2;     // negative days (DayAcc)
     unsigned n_neg;
     unsigned gap_bar, gap_minutes;   // calendar clock of a glued series (b200bt_sweep_config); gap_bar = ~0u: none
@@ -116,11 +112,6 @@ __device__ __forceinline__ double record_pnl(bool active, unsigned w, float pf, 
 static __device__ __noinline__ void batch_core(WarpAcc* __restrict__ acc, int cnt, unsigned w, float pf, unsigned w_carry,
                                         float p_carry, long long minute0, int bar_minutes, int64_t ev_cap) {
     const int lane = threadIdx.x & 31;
-#ifdef B200BT_SW_NOBATCH   // timing experiment only: skip the batch arithmetic
-    if (lane == 0) acc->n_events += cnt;
-    __syncwarp();
-    return;
-#endif
     const bool active = lane < cnt;
     float p_prev = __shfl_up_sync(FULL, pf, 1);
     unsigned w_prev = __shfl_up_sync(FULL, w, 1);
@@ -176,13 +167,6 @@ static __device__ __noinline__ void batch_core(WarpAcc* __restrict__ acc, int cn
     // calendar day of a record, relative to bar 0's day (32-bit: the host checks N*bar_minutes < 2^31 - 1440)
     const int day = active ? (int)(((unsigned)minute0 + bar * (unsigned)bar_minutes + (bar >= acc->gap_bar ? acc->gap_minutes : 0u)) / 1440u) : 0;
     DayAcc da{acc->pivot, acc->s1, acc->s2, acc->n_days, acc->pivot_set, acc->npivot, acc->ns1, acc->ns2, acc->n_neg};
-    const int hold_first = acc->hold_first;
-    int first_done = acc->first_done, first_id = acc->first_day;
-    double first_sum = acc->first_sum;
-    auto finish_day = [&](int id, double x) {
-        if (hold_first && !first_done) { first_done = 1; first_id = id; first_sum = x; }
-        else day_complete(da, x);
-    };
     const int day_valid = acc->day_valid;
     const int day_cur = (int)acc->day_cur;
     double day_sum = acc->day_sum;
@@ -213,11 +197,11 @@ static __device__ __noinline__ void batch_core(WarpAcc* __restrict__ acc, int cn
         unsigned done = __ballot_sync(FULL, tail && !last_seg_tail);
         // ... plus the carried day when the batch starts on a later day;
         // fold in time order (carry first, then lanes ascending)
-        if (day_valid && !merge_carry) finish_day(day_cur, day_sum);
+        if (day_valid && !merge_carry) day_complete(da, day_sum);
         while (done) {
             const int j = __ffs(done) - 1;
             done &= done - 1;
-            finish_day(__shfl_sync(FULL, day, j), shfl_d(x, j));
+            day_complete(da, shfl_d(x, j));
         }
         day_sum = shfl_d(seg, cnt - 1);
     }
@@ -242,7 +226,6 @@ static __device__ __noinline__ void batch_core(WarpAcc* __restrict__ acc, int cn
         acc->pivot = da.pivot; acc->s1 = da.s1; acc->s2 = da.s2; acc->n_days = da.n_days; acc->pivot_set = da.pivot_set;
         acc->npivot = da.npivot; acc->ns1 = da.ns1; acc->ns2 = da.ns2; acc->n_neg = da.n_neg;
         acc->day_sum = day_sum; acc->day_cur = last_day; acc->day_valid = 1;
-        acc->first_done = first_done; acc->first_day = first_id; acc->first_sum = first_sum;
         acc->hash ^= ((unsigned long long)hhi << 32) | hlo;
         acc->n_events = n_events + cnt;
     }
@@ -354,8 +337,6 @@ __device__ __forceinline__ void init_acc(WarpAcc& a, const b200bt_individual& iv
     a.ev_out = ev_out;
     a.n_win = a.n_loss = a.n_days = a.n_events = 0;
     a.day_valid = a.pivot_set = 0;
-    a.hold_first = a.first_done = a.first_day = 0;
-    a.first_sum = 0.0;
     a.npivot = a.ns1 = a.ns2 = 0.0;
     a.n_neg = 0;
 }
@@ -380,9 +361,6 @@ __device__ __forceinline__ void cp_async16(float* smem_dst, const float* gmem_sr
 __device__ __forceinline__ void cp_async4(float* smem_dst, const float* gmem_src) {
     asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"((unsigned)__cvta_generic_to_shared(smem_dst)), "l"(gmem_src) : "memory");
 }
-__device__ __forceinline__ void cp_async8(void* smem_dst, const void* gmem_src) {
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"((unsigned)__cvta_generic_to_shared(smem_dst)), "l"(gmem_src) : "memory");
-}
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 template <int N_>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N_) : "memory"); }
@@ -391,9 +369,6 @@ __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_gr
 __device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(unsigned long long* bar, unsigned count) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_inval(unsigned long long* bar) {
-    asm volatile("mbarrier.inval.shared::cta.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 __device__ __forceinline__ void mbar_fence_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
 __device__ __forceinline__ void mbar_arrive_expect_tx(unsigned long long* bar, unsigned bytes) {

@@ -326,7 +326,29 @@ def _flag_slot() -> torch.Tensor:
     return _pinned_flags()[i]
 
 
-class ChunkPlan:
+class _SweepPlan:
+    """What both time-chunked plans hold besides their schedule: the event pool, the workspace, the lanes' fallback flags
+    and a slot of the pinned flag table."""
+
+    def _allocate(self, pred: np.ndarray, n_symbols: int, device, pool_scale: float, pool_blocks: Optional[int],
+                  workspace: Optional[torch.Tensor], workspace_bytes) -> None:
+        """`workspace_bytes(pool_blocks)` sizes the workspace; `workspace` may be shared between the plans of successive
+        slices (DEFERRED: the caller assigns it)."""
+        # every segment owns at least one block, and a repaired segment abandons its first chain
+        self.pred_blocks = float(pred.sum()) * n_symbols / 256
+        self.pool_blocks = int(pool_scale * self.pred_blocks) + 2 * self.n_seg * n_symbols + 1024
+        if pool_blocks is not None:
+            self.pool_blocks = int(pool_blocks)
+        self.ws_bytes = int(workspace_bytes(self.pool_blocks))
+        if workspace is not None and workspace.numel() >= self.ws_bytes:
+            self.workspace = workspace
+        else:
+            self.workspace = None if workspace is DEFERRED else torch.empty(self.ws_bytes, dtype=torch.uint8, device=device)
+        self.invalid = torch.zeros((self.pop, n_symbols), dtype=torch.uint8, device=device)
+        self.overflow = _flag_slot()
+
+
+class ChunkPlan(_SweepPlan):
     """Host-side plan of the time-chunked sweep for one population (device tensors inside)."""
 
     def __init__(self, population: List[Dict], n_bars: int, n_symbols: int, device, target_events: int = 16384,
@@ -337,7 +359,7 @@ class ChunkPlan:
         plan are slice-relative); `workspace` may be shared between the plans of successive slices; `pred` =
         predicted_events(population, n_bars) when the caller already has it."""
         pop = len(population)
-        self.lo = int(lo)
+        self.lo, self.pop = int(lo), pop
         pred = predicted_events(population, n_bars) if pred is None else np.asarray(pred, dtype=np.float64)
         kmax = max(1, min(max_chunks, n_bars // max(8 * warm, 2048)))
         k = np.clip(np.ceil(pred / target_events), 1, kmax).astype(np.int32)
@@ -355,25 +377,15 @@ class ChunkPlan:
                 row += 1
         self.warm = int(warm)
         self.max_repair_rounds = int(max_repair_rounds)
-        self.pred_blocks = float(pred.sum()) * n_symbols / 256
-        self.pool_blocks = int(pool_scale * self.pred_blocks) + 2 * self.n_seg * n_symbols + 1024
-        if pool_blocks is not None:
-            self.pool_blocks = int(pool_blocks)
         self.items = torch.from_numpy(items).to(device)
         self.seg_base_dev = torch.from_numpy(self.seg_base).to(device)
         self.n_chunks_dev = torch.from_numpy(self.n_chunks).to(device)
         self.order_dev = torch.from_numpy(self.order).to(device)
-        self.ws_bytes = int(_lib.load().b200bt_sweep_chunked_workspace_bytes(self.pool_blocks, n_symbols, self.n_seg))
-        if workspace is not None and workspace.numel() >= self.ws_bytes:
-            self.workspace = workspace
-        else:
-            self.workspace = None if workspace is DEFERRED else torch.empty(self.ws_bytes, dtype=torch.uint8, device=device)
-        self.invalid = torch.zeros((pop, n_symbols), dtype=torch.uint8, device=device)
-        self.overflow = _flag_slot()
-        self.pop = pop
+        self._allocate(pred, n_symbols, device, pool_scale, pool_blocks, workspace,
+                       lambda blocks: _lib.load().b200bt_sweep_chunked_workspace_bytes(blocks, n_symbols, self.n_seg))
 
 
-class TilePlan:
+class TilePlan(_SweepPlan):
     """Host-side plan of the thread-per-lane sweep (b200bt_sweep_tiled) for one population slice: every
     individual gets the same K time chunks, chosen so that the CTAs fill whole waves of the GPU."""
 
@@ -413,20 +425,10 @@ class TilePlan:
         # 0 = no repair, 1 = the bounded pass on the critical path, 2 = that and the unbounded pass beside the metrics
         self.max_repair_rounds = int(max_repair_rounds) if max_repair_rounds is not None else 2
         self.n_seg = pop * self.K
-        # every segment owns at least one block, and a repaired segment abandons its first chain
-        self.pred_blocks = float(pred.sum()) * n_symbols / 256
-        self.pool_blocks = int(pool_scale * self.pred_blocks) + 2 * self.n_seg * n_symbols + 1024
-        if pool_blocks is not None:
-            self.pool_blocks = int(pool_blocks)
         self.order = np.ascontiguousarray(self.slots[self.slots >= 0])      # individuals in dispatch order
         self.slots_dev = torch.from_numpy(np.concatenate([self.slots, self.order])).to(device)     # [slots | order]
-        self.ws_bytes = int(_lib.load().b200bt_sweep_tiled_workspace_bytes(self.pool_blocks, n_symbols, pop, self.K))
-        if workspace is not None and workspace.numel() >= self.ws_bytes:
-            self.workspace = workspace
-        else:
-            self.workspace = None if workspace is DEFERRED else torch.empty(self.ws_bytes, dtype=torch.uint8, device=device)
-        self.invalid = torch.zeros((pop, n_symbols), dtype=torch.uint8, device=device)
-        self.overflow = _flag_slot()
+        self._allocate(pred, n_symbols, device, pool_scale, pool_blocks, workspace,
+                       lambda blocks: _lib.load().b200bt_sweep_tiled_workspace_bytes(blocks, n_symbols, pop, self.K))
 
 
 WARP_RSI_ROWS = 2       # distinct RSI rows the machines of one warp may read (csrc/sweep_chunked.cu LS_RSI_ROWS)
@@ -506,14 +508,8 @@ class PopulationSweep:
         mode: "fused" (one warp per lane, serial in time), "chunked" (expensive lanes split into verified
         time chunks, one warp per chunk), "tiled" (every lane split into the same K verified chunks, one THREAD
         per chunk; csrc/sweep_chunked.cu) or "auto" (tiled from 131072 bars up, fused below)."""
-        self.market = market
-        self.periods = sorted(set(int(p) for p in rsi_periods))
-        self.period_row = {p: i for i, p in enumerate(self.periods)}
-        goals = optimization_goals or DEFAULT_GOALS
-        primary, mask = _lib.score_codes(goals, advanced=score_on_advanced)
-        self.cfg = _lib.SweepConfig(initial_capital=float(initial_capital), minute0=market.minute0,
-                                    bar_minutes=market.bar_minutes, primary=primary, secondary_mask=mask, variant=0)
-        self.event_cap = int(event_cap)
+        self._configure(market, sorted(set(int(p) for p in rsi_periods)), optimization_goals, initial_capital, event_cap,
+                        mode, chunk_options, score_on_advanced)
         # timeframes (minutes per bar, the first one = the market's own clock): BASELINE configs[3] evaluates the RSI rule on
         # 1m / 5m / 15m indicators (recipe: services/market_monitor_service.py:219-301); the bank then holds one block of rows
         # per timeframe, each higher-timeframe RSI brought back to the base clock by "last completed bar", and the gene
@@ -522,12 +518,21 @@ class PopulationSweep:
         if self.timeframes[0] != market.bar_minutes or any(k % market.bar_minutes for k in self.timeframes):
             raise ValueError("timeframes must start with the market's own bar spacing and be multiples of it")
         self.bank = self._bank_behind_the_upload(market) if len(self.timeframes) == 1 else self._multi_timeframe_bank(market)
+
+    def _configure(self, market: MarketData, periods: List[int], optimization_goals: Optional[Dict], initial_capital: float,
+                   event_cap: int, mode: str, chunk_options: Optional[Dict], score_on_advanced: bool) -> None:
+        self.market = market
+        self.periods = periods
+        self.period_row = {p: i for i, p in enumerate(self.periods)}
+        goals = optimization_goals or DEFAULT_GOALS
+        primary, mask = _lib.score_codes(goals, advanced=score_on_advanced)
+        self.cfg = _lib.SweepConfig(initial_capital=float(initial_capital), minute0=market.minute0,
+                                    bar_minutes=market.bar_minutes, primary=primary, secondary_mask=mask, variant=0)
+        self.event_cap = int(event_cap)
         self.mode, self.chunk_min_bars, self.chunk_options = mode, 131072, dict(chunk_options or {})
-        self._stats = None
-        self._events = None
+        self._stats = self._events = None
         self._pop = 0
-        self._pinned_in = None
-        self._pinned_out = None
+        self._pinned_in = self._pinned_out = None
 
     def _bank_behind_the_upload(self, market: MarketData) -> torch.Tensor:
         """RSI bank of the market.  While the close prices are still arriving in quarter copies (MarketData from a
@@ -575,21 +580,11 @@ class PopulationSweep:
         """Sweep over a caller-supplied RSI bank [S][P][N] (e.g. the 'rsi' field of the reference's
         market-data points) instead of one computed from the close prices."""
         self = cls.__new__(cls)
-        self.market = market
-        self.periods = [int(p) for p in periods]
-        self.period_row = {p: i for i, p in enumerate(self.periods)}
-        goals = optimization_goals or DEFAULT_GOALS
-        primary, mask = _lib.score_codes(goals, advanced=score_on_advanced)
-        self.cfg = _lib.SweepConfig(initial_capital=float(initial_capital), minute0=market.minute0,
-                                    bar_minutes=market.bar_minutes, primary=primary, secondary_mask=mask, variant=0)
-        self.event_cap = int(event_cap)
+        self._configure(market, [int(p) for p in periods], optimization_goals, initial_capital, event_cap, mode, None,
+                        score_on_advanced)
         self.timeframes = (market.bar_minutes,)
         assert bank.is_cuda and bank.dtype == torch.float32 and tuple(bank.shape) == (market.S, len(self.periods), market.N)
         self.bank = bank.contiguous()
-        self.mode, self.chunk_min_bars, self.chunk_options = mode, 131072, {}
-        self._stats = self._events = None
-        self._pop = 0
-        self._pinned_in = self._pinned_out = None
         return self
 
     # -- device-side evaluation (inputs already resident) -------------------
@@ -610,11 +605,7 @@ class PopulationSweep:
             return
         m = self.market
         self._last_plans = []
-        if self._stats is None or self._pop != pop:
-            self._stats = torch.empty((pop, m.S, _lib.LANE_STATS_WORDS), dtype=torch.float64, device=m.device)
-            self._events = (torch.zeros((pop, m.S, self.event_cap), dtype=torch.int32, device=m.device)
-                            if self.event_cap else None)
-            self._pop = pop
+        self._ensure_buffers(pop)
         with torch.cuda.device(m.device):
             st = _lib.current_stream()
             _lib.call("b200bt_sweep", m.close.data_ptr(), _lib.ld(m.close), self.bank.data_ptr(),
